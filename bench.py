@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the search hot path (BASELINE.json: QPS, 1Mx960 Flat L2 kNN).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA kernels)
+    python bench.py [...] --dump-outputs DIR                        also write the last timed step's results as .npy
     python bench.py --impl reference [...]                          CPU arm: the oracle (reference
                                                                     semantics restated in C++; the Rust
                                                                     crate cannot be built in this image)
@@ -46,7 +47,34 @@ def parse():
     ap.add_argument("--cpu-queries", type=int, default=0, help="CPU sample size (0 = 2 x cores, <= 128)")
     ap.add_argument("--no-other-configs", action="store_true",
                     help="skip the IVF (configs[2]) and PQ (configs[3]) legs that follow the headline measurement at N=1")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64 << 20  # --dump-outputs: bound on all written arrays together
+
+
+def dump_outputs(out_dir, ids, dist, counts):
+    """The search results of the last timed step, as the caller of the timed path receives them, as DIR/<name>.npy:
+    ids and counts in float64 (exact below 2^53; an unfilled id slot reads -1), distances in float32. When the whole
+    batch is larger than DUMP_BYTES, a fixed seeded sample of the queries is written; query_rows.npy always names the
+    query rows written, so that two builds can be compared output for output."""
+    ids = np.asarray(ids).astype(np.int64).astype(np.float64)
+    dist = np.asarray(dist, np.float32)
+    counts = np.asarray(counts).astype(np.float64)
+    nq, k = ids.shape
+    rows = np.arange(nq)
+    per_query = k * (8 + 4) + 8 + 8
+    if nq * per_query > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(nq, DUMP_BYTES // per_query, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("ids", ids[rows]), ("dist", dist[rows]), ("counts", counts[rows]),
+                    ("query_rows", rows.astype(np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_fixtures():
@@ -301,7 +329,9 @@ def run_reference(args):
     import torch
     base = synth(base1000, 0, args.n, 42, dev).cpu().numpy()
     q = synth(test1000, 0, nqs, 43, dev).cpu().numpy()
-    qps, dt, _ = cpu_arm(base, q, args.k, cores, max(1, args.steps), min(args.warmup, 1))
+    qps, dt, res = cpu_arm(base, q, args.k, cores, args.steps, min(args.warmup, 1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *res)
     line = {
         "impl": "reference", "metric": "QPS, exact Flat L2 kNN", "value": qps, "unit": "queries/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt * 1e3,
@@ -551,6 +581,8 @@ def run_ours_multi(args):
         "tensor_path": stats, "host_wall_ms_per_step": wall / args.steps * 1e3, "nccl_multiprocess": nccl,
         "other_configs": other,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *res)
     print(json.dumps(line), flush=True)
     dist.destroy_process_group()
 
@@ -847,6 +879,8 @@ def run_ours(args):
     }
     if idx.phase_ms.get("calls"):  # VDB_PHASE_TIMING=1: per-phase device time of the sharded search (rank 0), ms per call
         line["phase_ms"] = {k_: round(v / idx.phase_ms["calls"], 4) for k_, v in idx.phase_ms.items() if k_ != "calls"}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *(t.cpu().numpy() for t in res))
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

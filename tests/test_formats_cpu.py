@@ -1,13 +1,10 @@
 """`not gpu`: on-disk formats either side of the path (bincode 1.3.3 layouts, raw vectors, fvecs, bench TOML)."""
-import os
 import struct
 
 import numpy as np
 import pytest
 
 from lab_1806_vec_db_b200 import formats as F
-
-REF = "/root/reference"
 
 
 def test_ground_truth_known_bytes():
@@ -84,16 +81,74 @@ def test_raw_and_fvecs(tmp_path, fixtures):
     assert (F.read_fvecs(tmp_path / "v.fvecs") == rows).all()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_reference_files_parse():
-    """The reference's own data/config files load through these readers."""
-    base = F.load_raw(f"{REF}/data/gist_1000.bin", 960)
+# BenchConfig / ResultList files in the reference's layout (examples/bench.rs:70-92, 312-368), carrying the settings and
+# published numbers of config/bench_10000_ivf.toml, config/bench_pq_240_hnsw.toml and data/t_bench_1e4.toml that
+# BASELINE.md and bench_configs.py quote
+BENCH_CONFIG = """label = "{label}"
+dist = "L2Sqr"
+gnd_path = "data/gnd_{label}.bin"
+index_cache = "data/index_{label}.bin"
+bench_output = "data/t_bench.toml"
+
+[ef.range]
+start = {ef0}
+end = {ef1}
+step = {step}
+
+[algorithm.{algo}]
+{body}
+{pq}
+[base]
+dim = 960
+data_type = "float32"
+data_path = "data/base.bin"
+
+[test]
+dim = 960
+data_type = "float32"
+data_path = "data/test.bin"
+"""
+RESULT_LIST = """title = "Bench (N=10000)"
+
+[[results]]
+label = "HNSW"
+ef = [120, 360]
+search_time = [0.0382, 0.0816]
+recall = [0.9927, 0.9990]
+
+[[results]]
+label = "HNSW+PQ"
+ef = [160, 360]
+search_time = [0.0369, 0.0632]
+recall = [0.9930, 0.9989]
+
+[[results]]
+label = "Flat+PQ"
+ef = [100, 200]
+search_time = [0.1271, 0.1360]
+recall = [0.9915, 0.9997]
+"""
+
+
+def test_reference_files_parse(tmp_path, fixtures):
+    """The reference's data file (rebuilt bit for bit from the fixture) and config / result files in its layout load
+    through these readers."""
+    import hashlib
+    F.save_raw(tmp_path / "gist_1000.bin", fixtures["base"])
+    assert hashlib.sha256((tmp_path / "gist_1000.bin").read_bytes()).hexdigest() == fixtures["base_sha256"]
+    base = F.load_raw(tmp_path / "gist_1000.bin", 960)
     assert base.shape == (1000, 960) and (base[50] == base[444]).all()
-    cfg = F.load_bench_config(f"{REF}/config/bench_10000_ivf.toml")
+    (tmp_path / "ivf.toml").write_text(BENCH_CONFIG.format(
+        label="IVF", ef0=8, ef1=24, step=4, algo="IVF", pq="",
+        body="k = 128\nk_means_size = 1000\nk_means_max_iter = 20\nk_means_tol = 1e-6"))
+    cfg = F.load_bench_config(tmp_path / "ivf.toml")
     assert cfg["ef_values"] == [8, 12, 16, 20, 24] and cfg["algorithm"]["IVF"]["k"] == 128 and cfg["dist"] == "l2sqr"
-    cfg = F.load_bench_config(f"{REF}/config/bench_pq_240_hnsw.toml")
+    (tmp_path / "pq.toml").write_text(BENCH_CONFIG.format(
+        label="HNSW+PQ", ef0=240, ef1=600, step=60, algo="HNSW", body="ef_construction = 200\nM = 16",
+        pq='[PQ]\ndist = "L2Sqr"\nn_bits = 4\nm = 240\nk_means_size = 10000\nk_means_max_iter = 20\nk_means_tol = 1e-6\n'))
+    cfg = F.load_bench_config(tmp_path / "pq.toml")
     assert cfg["PQ"]["m"] == 240 and cfg["ef_values"] == list(range(240, 601, 60))
-    res = F.load_result_list(open(f"{REF}/data/t_bench_1e4.toml").read())
+    res = F.load_result_list(RESULT_LIST)
     assert [r["label"] for r in res["results"]][:2] == ["HNSW", "HNSW+PQ"]
     text = F.dump_result_list(res["title"], res["results"])
     again = F.load_result_list(text)

@@ -180,6 +180,52 @@ def test_bench_reference_arm_contract():
     assert other.returncode == 0 and other.stdout.strip() == ""
 
 
+def test_bench_dump_outputs_are_the_timed_results_and_repeat(tmp_path):
+    """`--dump-outputs DIR`: the last timed step's ids / distances / counts as float .npy files; the same arguments give
+    the same inputs, so two runs write the same arrays (here through the CPU arm, checked against the oracle)."""
+    import oracle as O
+    import bench
+    runs = []
+    for i in range(2):
+        out = tmp_path / f"run{i}"
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--n", "20000", "--nq", "64",
+               "--k", "10", "--steps", "1", "--warmup", "0", "--cpu-queries", "4", "--dump-outputs", str(out)]
+        r = subprocess.run(cmd, capture_output=True, text=True, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        runs.append({n: np.load(out / f"{n}.npy") for n in ("ids", "dist", "counts", "query_rows")})
+    a, b = runs
+    for n in a:
+        assert a[n].dtype in (np.float32, np.float64) and a[n].tobytes() == b[n].tobytes(), n
+    assert a["ids"].shape == a["dist"].shape == (4, 10) and a["query_rows"].tolist() == [0, 1, 2, 3]
+    base1000, test1000 = bench.load_fixtures()
+    base = bench.synth(base1000, 0, 20000, 42, "cpu").numpy()
+    q = bench.synth(test1000, 0, 4, 43, "cpu").numpy()
+    wi, wd, wc = O.flat_knn(base, q, 10, "l2sqr")
+    assert (a["ids"] == wi).all() and (a["dist"] == wd).all() and (a["counts"] == wc).all()
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=600)
+    assert r.returncode == 2 and "--steps" in r.stderr                      # no run without a timed step
+
+
+def test_bench_dump_outputs_sample_a_large_batch(tmp_path):
+    """Beyond 64 MB in all, a fixed seeded sample of query rows is written, the same one every time."""
+    import bench
+    nq, k = 70_000, 100
+    ids = np.arange(nq * k, dtype=np.int64).reshape(nq, k)
+    dist = np.arange(nq * k, dtype=np.float32).reshape(nq, k)
+    counts = np.full(nq, k, np.int32)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), ids, dist, counts)
+    total = sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a"))
+    assert total <= bench.DUMP_BYTES + 4 * 4096                                          # + the .npy headers
+    rows = np.load(tmp_path / "a" / "query_rows.npy").astype(np.int64)
+    assert 0 < len(rows) < nq and (np.diff(rows) > 0).all()
+    assert (np.load(tmp_path / "a" / "ids.npy") == ids[rows]).all()
+    assert (np.load(tmp_path / "a" / "dist.npy") == dist[rows]).all()
+    for f in os.listdir(tmp_path / "a"):
+        assert (tmp_path / "a" / f).read_bytes() == (tmp_path / "b" / f).read_bytes(), f
+
+
 # ---- rand_compat: the reference's random stream restated (rand 0.8.5 StdRng = ChaCha12) -------------------------------
 def test_chacha_core_matches_the_published_keystreams():
     """Zero key, zero nonce, block 0: the keystream vectors published for ChaCha8 / ChaCha12 / ChaCha20 (the eSTREAM /
