@@ -276,6 +276,14 @@ int vdb_decode_keys_dev(const uint64_t* d_keys, uint32_t nq, uint32_t k, uint64_
  * from the measured per-row / per-query operand errors. d_queries: device [nq, dim] of the dataset dtype. Synchronous. */
 int vdb_debug_gemm_scores_dev(const vdb_dataset* ds, const void* d_queries, uint32_t nq, uint32_t row_stride,
                               int kind, uint64_t* d_out_keys, void* stream);
+/* Bounds of the tensor-core PQ filter (4-bit L2Sqr tables of >= 65536 rows): for every (query, row) of the table,
+ * d_lower[q * n + row] = the filter's lower bound S' of the exact ADC value (a row is dropped iff S' > tau_q) and
+ * d_upper[q * n + row] = the sample pass's upper bound U of it, from the kernels and constants of the search.
+ * path 0 = one-hot contraction over the BF16 lookup tables, 1 = contraction over decoded rows (sub-vectors of 4 dims;
+ * its score is mapped back to the smallest tau_q at which the filter keeps the row). d_queries: device [nq, dim] of
+ * the table's dtype; d_lower / d_upper: device [nq, n] f32. Synchronous. */
+int vdb_debug_pq_bounds_dev(const vdb_pq* pq, const void* d_queries, uint32_t nq, int path, float* d_lower,
+                            float* d_upper, void* stream);
 /* Side arrays of the tensor-core path of an (unsharded) dataset, built lazily by the first batched search and dropped on
  * mutation: operand kind (-1 = not built, 0 = TF32: the fp32 rows in place, 1 = FP16 copy), its power-of-two scale, the
  * mean row norm / mean operand-error norm, and the HBM bytes they occupy (FP16 kind: 2 bytes per element + 12 bytes per

@@ -105,6 +105,7 @@ SIGNATURES = {
     "vdb_merge_keys_to_keys_dev": (i32, [vp, u32, u32, u32, vp, vp]),
     "vdb_decode_keys_dev": (i32, [vp, u32, u32, vp, vp, vp, vp]),
     "vdb_debug_gemm_scores_dev": (i32, [vp, vp, u32, u32, i32, vp, vp]),
+    "vdb_debug_pq_bounds_dev": (i32, [vp, vp, u32, i32, vp, vp, vp]),
     "vdb_dataset_operand_info": (i32, [vp, vp, vp, vp, vp, vp]),
     "vdb_dataset_drop_side_arrays": (i32, [vp]),
     "vdb_flat_gemm_fallbacks": (u64, []),

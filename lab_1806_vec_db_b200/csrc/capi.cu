@@ -792,6 +792,25 @@ int vdb_debug_gemm_scores_dev(const vdb_dataset* ds, const void* d_queries, uint
         vdb::flat_gemm_store(ds, d_queries, nq, row_stride, kind, d_out_keys, (cudaStream_t)stream);
     });
 }
+int vdb_debug_pq_bounds_dev(const vdb_pq* pq, const void* d_queries, uint32_t nq, int path, float* d_lower, float* d_upper,
+                            void* stream) {
+    return guarded([&] {
+        VDB_REQUIRE(pq && d_queries && d_lower && d_upper && nq > 0, "NULL argument");
+        VDB_REQUIRE(path == 0 || path == 1, "path must be 0 (one-hot) or 1 (decoded)");
+        if (!pq->shards.empty()) vdb::fail(VDB_EUNSUPPORTED, "vdb_debug_pq_bounds_dev: call it on the shards' tables");
+        DeviceGuard g(pq->device);
+        cudaStream_t st = (cudaStream_t)stream;
+        if (path == 1) {
+            vdb::pq_dec_bounds(pq, d_queries, nq, d_lower, d_upper, st);
+            return;
+        }
+        VDB_REQUIRE(vdb::pq_tensor_supported(pq, UINT32_MAX), "one-hot PQ contraction: unsupported table");
+        vdb::DevBuf lut((size_t)nq * pq->m * pq->kc * 4, st), qc((size_t)nq * 4, st);
+        vdb::pq_lut(pq, d_queries, nq, lut.as<float>(), qc.as<float>(), st);
+        vdb::pq_tensor_bounds(pq, lut.as<float>(), nq, d_lower, d_upper, st);
+        VDB_CUDA(cudaStreamSynchronize(st));
+    });
+}
 int vdb_dataset_operand_info(const vdb_dataset* ds, int* kind, float* scale, float* mean_norm, float* mean_ex,
                              uint64_t* side_bytes) {
     return guarded([&] {

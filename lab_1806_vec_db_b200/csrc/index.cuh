@@ -183,6 +183,8 @@ void pq_dec_sample(const vdb_pq* pq, void* ctx, uint32_t nq, float* d_all, cudaS
 void pq_dec_filter(const vdb_pq* pq, void* ctx, const float* d_lut, uint32_t nq, const float* d_tau, uint32_t id_base,
                    uint32_t* d_cnt, uint64_t* d_cand, uint32_t cap, cudaStream_t st);
 void pq_dec_destroy(vdb_pq* pq);
+// test hook: lower bound of the filter / upper bound of the sample pass of every (query, row), [nq][n] each
+void pq_dec_bounds(const vdb_pq* pq, const void* d_queries, uint32_t nq, float* d_lower, float* d_upper, cudaStream_t st);
 // exact ADC (reference arithmetic) of coarse candidate rows; survivors with adc <= tau become keys (pq_gemm.cu)
 void pq_exact_candidates(const vdb_pq* pq, const float* d_lut, const float* d_tau, uint32_t nq, const uint32_t* d_ccnt,
                          const uint32_t* d_ccand, uint32_t ccap, uint32_t id_base, uint32_t* d_cnt, uint64_t* d_cand,
@@ -191,6 +193,7 @@ void pq_tensor_lut(const vdb_pq* pq, const float* d_lut, uint32_t nq, DevBuf& lu
 void pq_tensor_sample(const vdb_pq* pq, const DevBuf& lut16, uint32_t nq, float* d_all, cudaStream_t st);
 void pq_tensor_filter(const vdb_pq* pq, const DevBuf& lut16, const float* d_lut, uint32_t nq, const float* d_tau, uint32_t id_base,
                       uint32_t* d_cnt, uint64_t* d_cand, uint32_t cap, cudaStream_t st);
+void pq_tensor_bounds(const vdb_pq* pq, const float* d_lut, uint32_t nq, float* d_lower, float* d_upper, cudaStream_t st);
 
 // flat_gemm.cu
 void flat_gemm_store(const vdb_dataset* ds, const void* d_queries, uint32_t nq, uint32_t row_stride, int kind,

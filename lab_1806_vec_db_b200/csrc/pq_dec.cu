@@ -29,6 +29,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
+#include <memory>
 #include <mutex>
 #include <vector>
 
@@ -69,7 +70,7 @@ struct PqDecParams {
     uint32_t* ccand;          // [nq][ccap] rows
     uint32_t ccap;
     uint32_t tiles_per_item, nrow_items, nqt;
-    float* all_out;           // MODE 0: [nq][n] upper bounds of the exact ADC values (sample pass)
+    float* all_out;           // MODE 0: [nq][n] upper bounds of the exact ADC values (sample pass); MODE 2: [nq][n] scores
     // MODE 1 output: one record per (row, chunk of 32 queries) with any passing score - the per-query candidate lists are
     // filled from the records by pq_dec_expand_kernel. (Appending to the per-query lists from the epilogue costs one
     // atomic round trip per passing score in divergent code: at 0.25 % passing scores the four epilogue warps needed
@@ -80,7 +81,7 @@ struct PqDecParams {
     uint32_t rec_cap;
 };
 
-// MODE 0: store an upper bound of every ADC value (sample pass), 1: filter
+// MODE 0: store an upper bound of every ADC value (sample pass), 1: filter, 2: store every filter score (test hook)
 template <int MODE>
 __global__ void __launch_bounds__(D_THREADS, 1) pq_dec_kernel(const __grid_constant__ CUtensorMap map_q, const PqDecParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -288,7 +289,10 @@ __global__ void __launch_bounds__(D_THREADS, 1) pq_dec_kernel(const __grid_const
                                 for (int jj = 0; jj < 4; ++jj) {
                                     const int j = j4 + jj;
                                     const float dot = __uint_as_float(v[j]);
-                                    if (MODE == 0) {
+                                    if (MODE == 2) {
+                                        const uint32_t q = q0 + c0 + j;
+                                        if (q < p.nq) p.all_out[(size_t)q * p.n + row] = fmaf(dv[jj], dot, fmaf(-bv[jj], xn, rr));
+                                    } else if (MODE == 0) {
                                         // upper bound of the reference's ADC value; a warp stores 32 consecutive rows of a query
                                         const uint32_t q = q0 + c0 + j;
                                         const float up = (fmaf(dv[jj], dot, fmaf(bv[jj], xn, rr)) + tv[jj]) * 1.00005f + 1e-30f;
@@ -507,13 +511,36 @@ __global__ void __launch_bounds__(256) pq_dec_query_kernel(const T* __restrict__
         qab[q] = (2.0f * qn1 + b) * ex_max;   // (coefficient of the decode error) x (its worst case over all code words)
     }
 }
+// MODE 1 threshold of the score for the ADC threshold tau (non-decreasing in tau)
+__device__ __forceinline__ float dec_score_threshold(float tau, float qsq, float qab) {
+    return tau * 1.00005f - qsq * 0.99995f + qab + 1e-30f;
+}
 // MODE 1 threshold of the score / MODE 0 additive constant of the upper bound
 __global__ void pq_dec_thresholds_kernel(const float* __restrict__ tau, const float* __restrict__ qsq, const float* __restrict__ qab,
                                          uint32_t nq, float* __restrict__ out) {
     const uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= nq) return;
-    if (tau) out[q] = tau[q] * 1.00005f - qsq[q] * 0.99995f + qab[q] + 1e-30f;
+    if (tau) out[q] = dec_score_threshold(tau[q], qsq[q], qab[q]);
     else out[q] = qsq[q] * 1.00005f + qab[q];
+}
+// test hook: filter score -> the smallest ADC threshold tau at which the filter keeps the row (its lower bound of the
+// ADC value in the units of the other paths): bisection over the ordered float bit patterns, the threshold being
+// non-decreasing in tau. NaN scores are kept at every threshold (-inf).
+__global__ void pq_dec_lower_kernel(float* __restrict__ v, uint32_t nq, uint64_t n, const float* __restrict__ qsq,
+                                    const float* __restrict__ qab) {
+    const uint64_t total = (uint64_t)nq * n;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t q = (uint32_t)(i / n);
+        const float sc = v[i];
+        uint32_t lo = f32_order_bits(__uint_as_float(0xff800000u)), hi = f32_order_bits(__uint_as_float(0x7f800000u));
+        if (!(sc > dec_score_threshold(f32_from_order_bits(lo), qsq[q], qab[q]))) hi = lo;
+        while (hi - lo > 1) {   // invariant: the row is dropped at lo, kept at hi
+            const uint32_t mid = lo + (hi - lo) / 2;
+            if (sc > dec_score_threshold(f32_from_order_bits(mid), qsq[q], qab[q])) lo = mid;
+            else hi = mid;
+        }
+        v[i] = f32_from_order_bits(hi);
+    }
 }
 
 struct PqDecQueries {
@@ -547,6 +574,10 @@ static void launch_dec(int mode, const vdb_pq* pq, const PqDecQueries& Q, uint32
         static std::atomic<size_t> configured[VDB_MAX_DEVICES];
         ensure_dyn_smem(pq_dec_kernel<0>, dec_smem_bytes(D_MAX_M), configured);
         pq_dec_kernel<0><<<grid, D_THREADS, smem, st>>>(map, p);
+    } else if (mode == 2) {
+        static std::atomic<size_t> configured[VDB_MAX_DEVICES];
+        ensure_dyn_smem(pq_dec_kernel<2>, dec_smem_bytes(D_MAX_M), configured);
+        pq_dec_kernel<2><<<grid, D_THREADS, smem, st>>>(map, p);
     } else {
         static std::atomic<size_t> configured[VDB_MAX_DEVICES];
         ensure_dyn_smem(pq_dec_kernel<1>, dec_smem_bytes(D_MAX_M), configured);
@@ -621,6 +652,25 @@ void pq_dec_filter(const vdb_pq* pq, void* ctx, const float* d_lut, uint32_t nq,
                                                                   rec_cap, nq, ccnt.as<uint32_t>(), ccand.as<uint32_t>(), ccap);
     VDB_LAUNCHED();
     pq_exact_candidates(pq, d_lut, d_tau, nq, ccnt.as<uint32_t>(), ccand.as<uint32_t>(), ccap, id_base, d_cnt, d_cand, cap, st);
+}
+
+// test hook: the filter's lower bound (pq_dec_lower_kernel) and the sample pass's upper bound of the ADC value of every
+// (query, row) of the table, [nq][n] each, from the same kernel and coefficients as pq_dec_filter / pq_dec_sample
+void pq_dec_bounds(const vdb_pq* pq, const void* d_queries, uint32_t nq, float* d_lower, float* d_upper, cudaStream_t st) {
+    VDB_REQUIRE(pq_dec_supported(pq, UINT32_MAX), "decoded PQ contraction: unsupported table");
+    const std::unique_ptr<PqDecQueries> ctx(static_cast<PqDecQueries*>(pq_dec_begin(pq, d_queries, nq, st)));
+    VDB_REQUIRE(ctx, "decoded PQ contraction: codebooks not representable in FP16");
+    auto& Q = *ctx;
+    pq_dec_thresholds_kernel<<<ceil_div(nq, 256u), 256, 0, st>>>(nullptr, Q.qsq.as<float>(), Q.qab.as<float>(), nq, Q.qt.as<float>());
+    VDB_LAUNCHED();
+    PqDecParams p{};
+    p.all_out = d_upper;
+    launch_dec(0, pq, Q, nq, pq->d_codes, pq->n, pq->d_dec_r, pq->d_dec_xn, p, st);
+    p.all_out = d_lower;
+    launch_dec(2, pq, Q, nq, pq->d_codes, pq->n, pq->d_dec_r, pq->d_dec_xn, p, st);
+    pq_dec_lower_kernel<<<(uint32_t)sm_count() * 8, 256, 0, st>>>(d_lower, nq, pq->n, Q.qsq.as<float>(), Q.qab.as<float>());
+    VDB_LAUNCHED();
+    VDB_CUDA(cudaStreamSynchronize(st));
 }
 
 }  // namespace vdb

@@ -4,8 +4,9 @@
 // d(q, row) = sum_g LUT_q[g][code(row, g)], flat_index.rs knn_pq) for large batches. The lookup is a dot product
 // with a ONE-HOT vector: adc(q, row) = < onehot(row), LUT_q > over K = m * 16 columns. The tensor cores evaluate it
 // in BF16 and only PRUNE: every LUT entry of an L2Sqr table is >= 0, so the BF16 rounding of the table is a RELATIVE
-// error (2^-9 per entry, one-hot entries are exact) and
-//     S' = S_bf16 * (1 - 2^-9 * 1.05 - m * 2^-21) - 1e-35  <=  adc_exact(q, row)
+// error (< 2^-8 per entry: BF16 keeps 8 significant bits, so round-to-nearest moves a value by up to half of its 2^-7
+// spacing; one-hot entries are exact) and
+//     S' = S_bf16 * (1 - 2^-8 * 1.05 - m * 2^-21) - 1e-35  <=  adc_exact(q, row)
 // holds for every pair. Rows with S' <= tau_q (tau_q: the exact-ADC threshold of the global-threshold scan, pq.cu)
 // become coarse candidates; their ADC value is then re-evaluated with the reference's arithmetic (sequential f32 sum
 // in group order) and the rows with adc <= tau_q go on exactly as in the FP32 scan — the candidate set is identical.
@@ -85,11 +86,16 @@ struct PqGemmParams {
     uint32_t* ccand;        // [nq][ccap] rows
     uint32_t ccap;
     uint32_t tiles_per_item, nrow_items, nqt;
-    float* all_out;         // MODE 0: [nq][n] upper bounds of the exact ADC values (sample pass)
+    float* all_out;         // MODE 0: [nq][n] upper bounds of the exact ADC values (sample pass); MODE 2: [nq][n] S'
     float up_factor;        // MODE 0: 1 + relative bound
 };
 
-// MODE 0: store every score (sample pass), 1: filter against tau. GG generator groups of 4 warps take the k-blocks
+// relative bound of the bf16 evaluation (see the top of the file)
+static float pq_rel_bound(uint32_t m) { return ldexpf(1.05f, -8) + (float)m * ldexpf(1.0f, -21); }
+// the filter's lower bound S' of the exact ADC value, from the fp32 accumulator of the contraction
+__device__ __forceinline__ float pq_filter_score(float acc, float factor) { return fmaf(acc, factor, -1e-35f); }
+
+// MODE 0: store every score (sample pass), 1: filter against tau, 2: store every S' of the filter (test hook). GG generator groups of 4 warps take the k-blocks
 // round-robin: one group's chain per k-block (wait -> LDS -> STS -> proxy fence -> arrive) is longer than the MMAs of a
 // k-block, so several chains have to be in flight.
 template <int MODE, int CTAS, int GG>
@@ -280,13 +286,14 @@ __global__ void __launch_bounds__(P_BASE_THREADS + 128 * GG, 1) pq_gemm_kernel(c
                     if (row_ok) {
 #pragma unroll
                         for (int j = 0; j < 32; ++j) {
-                            if (MODE == 0) {
+                            if (MODE != 1) {
                                 // a warp stores 32 consecutive rows of one query: 128-byte segments
                                 const uint32_t q = q0 + c0 + j;
-                                if (q < p.nq) p.all_out[(size_t)q * p.n + row] = __uint_as_float(v[j]) * p.up_factor;
+                                const float x = __uint_as_float(v[j]);
+                                if (q < p.nq) p.all_out[(size_t)q * p.n + row] = MODE == 0 ? x * p.up_factor : pq_filter_score(x, p.factor);
                                 continue;
                             }
-                            const float s = fmaf(__uint_as_float(v[j]), p.factor, -1e-35f);
+                            const float s = pq_filter_score(__uint_as_float(v[j]), p.factor);
                             if (!(s > tau_s[c0 + j])) {  // also keeps NaN (the exact re-evaluation decides)
                                 const uint32_t q = q0 + c0 + j;
                                 if (q < p.nq) {
@@ -464,7 +471,7 @@ static void launch_pq_gemm(const vdb_pq* pq, const DevBuf& lut16, uint32_t nq, c
 void pq_tensor_sample(const vdb_pq* pq, const DevBuf& lut16, uint32_t nq, float* d_all, cudaStream_t st) {
     PqGemmParams p{};
     p.all_out = d_all;
-    p.up_factor = 1.0f + (ldexpf(1.05f, -9) + (float)pq->m * ldexpf(1.0f, -21));
+    p.up_factor = 1.0f + pq_rel_bound(pq->m);
     launch_pq_gemm<0>(pq, lut16, nq, pq->d_sample, pq->sample_n, p, st);
 }
 
@@ -478,13 +485,28 @@ void pq_tensor_filter(const vdb_pq* pq, const DevBuf& lut16, const float* d_lut,
     VDB_CUDA(cudaMemsetAsync(ccnt.p, 0, (size_t)nq * 4, st));
     PqGemmParams p{};
     p.tau = d_tau;
-    p.factor = 1.0f - (ldexpf(1.05f, -9) + (float)pq->m * ldexpf(1.0f, -21));
+    p.factor = 1.0f - pq_rel_bound(pq->m);
     p.ccnt = ccnt.as<uint32_t>();
     p.ccand = ccand.as<uint32_t>();
     p.ccap = ccap;
     launch_pq_gemm<1>(pq, lut16, nq, pq->d_codes, pq->n, p, st);
     (void)tab;
     pq_exact_candidates(pq, d_lut, d_tau, nq, ccnt.as<uint32_t>(), ccand.as<uint32_t>(), ccap, id_base, d_cnt, d_cand, cap, st);
+}
+
+// test hook: the filter's S' (d_lower) and the sample pass's upper bound (d_upper) of every (query, row) of the table,
+// [nq][n] each, from the same kernel and constants as pq_tensor_filter / pq_tensor_sample
+void pq_tensor_bounds(const vdb_pq* pq, const float* d_lut, uint32_t nq, float* d_lower, float* d_upper, cudaStream_t st) {
+    DevBuf lut16;
+    pq_tensor_lut(pq, d_lut, nq, lut16, st);
+    PqGemmParams p{};
+    p.all_out = d_upper;
+    p.up_factor = 1.0f + pq_rel_bound(pq->m);
+    launch_pq_gemm<0>(pq, lut16, nq, pq->d_codes, pq->n, p, st);
+    p = PqGemmParams{};
+    p.all_out = d_lower;
+    p.factor = 1.0f - pq_rel_bound(pq->m);
+    launch_pq_gemm<2>(pq, lut16, nq, pq->d_codes, pq->n, p, st);
 }
 
 void pq_exact_candidates(const vdb_pq* pq, const float* d_lut, const float* d_tau, uint32_t nq, const uint32_t* d_ccnt,
