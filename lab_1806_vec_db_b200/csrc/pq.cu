@@ -9,6 +9,10 @@
 //
 // Codes, lookup tables and ADC distances are bit-exact: every sum is one thread's sequential f32 chain
 // in the reference's order (group order, low nibble = even group first) with unfused multiply/add.
+// Pinned by tests/test_index_gpu.py (4-bit m = 240 / 7, 8-bit m = 5) and tests/test_pq_paths_gpu.py: 8-bit codes with
+// m % 4 != 0 through every pq_adc_scan_kernel<NQ = 1/2/4, 8, *, LUT_SMEM = true> and <1, 8, *, false>, u8 rows,
+// 4-bit sub-vectors longer than ENC_MAXL (pq_encode_kernel), <1, 4, L2SQR, false> at m = 3000, and the top-k of
+// the per-CTA scan under maximal candidate pressure.
 // HBM layout of the codes for the scan: blocks of 32 rows, word-major ([block][word][lane]) so a warp's
 // load of one code word for its 32 rows is a single coalesced 128-byte request; one lane owns one row, all
 // lanes look up the SAME group at the same time, so the 16-entry LUT row is read conflict free.
