@@ -229,6 +229,28 @@ int vdb_ivf_knn_dev(const vdb_dataset* ds, const vdb_ivf* ivf, const void* d_que
                     uint32_t k, uint32_t n_probes, uint64_t* d_ids, float* d_dist, uint32_t* d_counts,
                     void* stream);
 
+/* ---- IVF + PQ ------------------------------------------------------------------------------- */
+/* IndexPQ::knn_pq on the IVF index. The reference has no IVF knn_pq; this library defines it as FlatIndex::knn_pq
+ * (src/index_algorithm/flat_index.rs:84-104) restricted to the rows of the n_probes nearest lists (find_n_nearest,
+ * src/distance/k_means.rs:174-191; n_probes clamped to nlist): the max(ef, k) smallest (ADC, id) over those rows in the
+ * reference's ADC arithmetic (src/distance/pq_table.rs:239-301), re-scored exactly, the k smallest (distance, id) kept
+ * (pq_resort, candidate_pair.rs:102-108); counts[q] = min(k, rows in the probed lists). Only the codes of the probed lists
+ * are scanned. With n_probes >= nlist the result is bit-identical to vdb_pq_knn on the same table. The first call with a
+ * table copies its codes into list order on the index (n * ceil(encoded_dim / 4) * 4 bytes; a call with another table
+ * replaces the copy). Errors (VDB_EINVAL, in this order): the index or the table was built for another vector set (a
+ * table must be rebuilt after add / delete), metric mismatch, n_probes == 0. On a row-sharded set vdb_ivf_knn_pq is one
+ * call over all shards (index and table built on that set). */
+int vdb_ivf_knn_pq(const vdb_dataset* ds, const vdb_ivf* ivf, const vdb_pq* pq, const void* queries, uint32_t nq, uint32_t k,
+                   uint32_t ef, uint32_t n_probes, uint64_t* ids, float* dist, uint32_t* counts);
+/* Device pointers. Like vdb_ivf_knn_dev it synchronises `stream` once: the probed lists are grouped on the host. */
+int vdb_ivf_knn_pq_dev(const vdb_dataset* ds, const vdb_ivf* ivf, const vdb_pq* pq, const void* d_queries, uint32_t nq,
+                       uint32_t k, uint32_t ef, uint32_t n_probes, uint64_t* d_ids, float* d_dist, uint32_t* d_counts,
+                       void* stream);
+/* The candidate stage alone (counterpart of vdb_pq_adc_keys_dev): d_keys [nq, kk] = the kk best (ADC, global id) packed
+ * keys per query over the probed lists, ascending, UINT64_MAX padded. Synchronises `stream` once. */
+int vdb_ivf_pq_adc_keys_dev(const vdb_dataset* ds, const vdb_ivf* ivf, const vdb_pq* pq, const void* d_queries, uint32_t nq,
+                            uint32_t kk, uint32_t n_probes, uint64_t* d_keys, void* stream);
+
 /* ---- tensor-core Flat path, phase by phase (row-sharded search: lab_1806_vec_db_b200/sharded.py) ---------
  * The single-GPU vdb_flat_knn runs these phases internally. Across shards the thresholds must be GLOBAL (else
  * every shard reranks its own ~750 candidates per query), so the phases are exported and the host inserts the
@@ -364,7 +386,7 @@ uint64_t vdb_launch_count(void);
  * kernels with CUDA events on the launching stream. vdb_prof_read synchronises the device, then
  * returns the accumulated milliseconds and launch count of kernel `name` since the last reset
  * (names: "flat_scan", "flat_gemm", "rerank", "merge", "pq_adc", "pq_encode", "ivf_scan",
- * "kmeans_assign", "pq_gemm", "pq_exact", "pq_lut", "pq_train", "hnsw_search", "hnsw_select", "hnsw_arrange"). */
+ * "kmeans_assign", "pq_gemm", "pq_exact", "pq_lut", "pq_train", "hnsw_search", "hnsw_select", "hnsw_arrange", "ivf_pq_scan"). */
 int vdb_prof_enable(int on);
 int vdb_prof_reset(void);
 int vdb_prof_read(const char* name, double* ms, uint64_t* launches);

@@ -92,6 +92,9 @@ SIGNATURES = {
     "vdb_ivf_lists": (i32, [vp, vp, vp]),
     "vdb_ivf_knn": (i32, [vp, vp, vp, u32, u32, u32, vp, vp, vp]),
     "vdb_ivf_knn_dev": (i32, [vp, vp, vp, u32, u32, u32, vp, vp, vp, vp]),
+    "vdb_ivf_knn_pq": (i32, [vp, vp, vp, vp, u32, u32, u32, u32, vp, vp, vp]),
+    "vdb_ivf_knn_pq_dev": (i32, [vp, vp, vp, vp, u32, u32, u32, u32, vp, vp, vp, vp]),
+    "vdb_ivf_pq_adc_keys_dev": (i32, [vp, vp, vp, vp, u32, u32, u32, vp, vp]),
     "vdb_tq_info": (i32, [vp, vp, vp, vp, vp]),
     "vdb_tq_j0": (u32, [u32, u64, u64]),
     "vdb_tq_begin_dev": (i32, [vp, vp, u32, vp, vp]),

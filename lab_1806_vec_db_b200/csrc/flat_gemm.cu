@@ -2211,7 +2211,7 @@ __global__ void ivf_sample_gather_kernel(const uint4* __restrict__ rows_lo, uint
     }
 }
 
-static std::mutex g_ivf_side_mu;
+std::mutex g_ivf_side_mu;
 static void ensure_ivf_side(const vdb_dataset* ds, const vdb_ivf* civf, cudaStream_t st) {
     const std::vector<uint64_t>& h_off = civf->h_off;
     vdb_ivf* ivf = const_cast<vdb_ivf*>(civf);

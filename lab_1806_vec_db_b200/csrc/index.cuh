@@ -1,5 +1,7 @@
 // index.cuh — device mirrors of PQTable / IVFIndex and the k-means / pair-distance launchers.
 #pragma once
+#include <memory>
+#include <mutex>
 #include <vector>
 
 #include "dataset.cuh"
@@ -7,6 +9,7 @@
 // device mirror of PQTable<T> (reference src/distance/pq_table.rs:116-137)
 struct vdb_pq {
     int device = 0;
+    uint64_t serial = 0;            // process-wide creation number (keys the list-ordered copy of the codes an IVF keeps)
     uint32_t dim = 0, m = 0, n_bits = 0, kc = 0, enc = 0;  // enc = encoded_dim (bytes per row)
     int dtype = VDB_F32, metric = VDB_L2SQR;
     uint64_t n = 0;
@@ -33,6 +36,7 @@ struct vdb_pq {
 
 // device mirror of IVFIndex<T> (reference src/index_algorithm/ivf_index.rs:34-47)
 struct vdb_tq;  // per-call query context of the tensor path (flat_gemm.cu)
+struct IvfPqCodes;  // one PQ table's codes in list order (ivf_pq.cu)
 
 struct vdb_ivf {
     int device = 0;
@@ -57,6 +61,9 @@ struct vdb_ivf {
     float* d_samp_colA = nullptr, *d_samp_rn = nullptr, *d_samp_ex = nullptr;
     std::vector<uint64_t> h_samp_off;  // [nlist+1]
     uint64_t samp_n = 0;
+    // lazily built by the first knn_pq call with a table (ivf_pq.cu), rebuilt when a call brings another table; a call
+    // holds its own reference, so a rebuild never frees codes a running scan reads
+    std::shared_ptr<const IvfPqCodes> pq_codes;
     std::vector<vdb_ivf*> shards;      // row-sharded parent (multi.cu): one index per shard, the arrays above stay empty
     const struct vdb_dataset* parent = nullptr;   // the sharded dataset it was built on
 };
@@ -93,6 +100,8 @@ vdb_pq* sharded_pq_create(const vdb_dataset* md, const void* h_codebooks, uint32
                           uint8_t* h_codes_out);
 void sharded_pq_knn(const vdb_dataset* md, const vdb_pq* pq, const void* queries, uint32_t nq, uint32_t k, uint32_t ef,
                     uint64_t* ids, float* dist, uint32_t* counts);
+void sharded_ivf_knn_pq(const vdb_dataset* md, const vdb_ivf* ivf, const vdb_pq* pq, const void* queries, uint32_t nq, uint32_t k,
+                        uint32_t ef, uint32_t n_probes, uint64_t* ids, float* dist, uint32_t* counts);
 
 // hnsw.cu
 vdb_hnsw* hnsw_build(const vdb_dataset* ds, uint32_t M, uint32_t ef_construction, const uint32_t* h_levels, uint32_t max_batch);
@@ -147,6 +156,9 @@ void pq_knn_keys(const vdb_dataset* ds, const vdb_pq* pq, const void* d_queries,
 
 void rerank_keys(const vdb_dataset* ds, const void* d_queries, uint32_t nq, const uint64_t* d_cand, uint32_t kk,
                  uint32_t k, uint64_t* d_keys, cudaStream_t st);
+// reference layout [n][enc] -> the scan's [ceil(n/32)][words][32] u32
+__global__ void pq_transpose_kernel(const uint8_t* __restrict__ codes, uint64_t n, uint32_t enc, uint32_t words,
+                                    uint32_t* __restrict__ out);
 
 // ivf.cu
 vdb_ivf* ivf_create(const vdb_dataset* ds, const void* h_centroids, uint32_t nlist, uint32_t* h_assign_out);
@@ -159,6 +171,38 @@ void ivf_list_major_subset(const vdb_dataset* ds, const vdb_ivf* ivf, const void
                            cudaStream_t st);
 void ivf_knn_keys(const vdb_dataset* ds, const vdb_ivf* ivf, const void* d_queries, uint32_t nq, uint32_t k,
                   uint32_t n_probes, uint64_t* d_keys, cudaStream_t st);
+extern std::mutex g_ivf_side_mu;   // guards the lazily built list-ordered arrays of every vdb_ivf
+__global__ void gather_bytes_rows_kernel(const uint8_t* __restrict__ src, uint32_t row_bytes, const uint32_t* __restrict__ idx,
+                                         uint32_t cnt, uint8_t* __restrict__ dst);
+// [nq][nprobe] keys (distance, list id) of the nprobe nearest lists per query, ascending: find_n_nearest (k_means.rs:174-191)
+DevBuf ivf_probe_keys(const vdb_dataset* ds, const vdb_ivf* ivf, const void* d_queries, uint32_t nq, uint32_t nprobe,
+                      cudaStream_t st);
+// Work items of the list-major batched scans: (list, up to `group` <= LQ queries that probe it, a range of the list's
+// positions). Query q's partial lists (one per item it is in; partial list index = item * group + query slot) are
+// plist[poff[q] .. poff[q + 1]). Ranges are multiples of `tile` positions, at least `min_range`, sized so that there are
+// enough items to fill the GPU a few times.
+constexpr int LQ = 8;
+struct IvfItem {
+    uint64_t row_begin;   // offset into members[]
+    uint32_t nrows;
+    uint32_t nq_valid;
+    uint32_t qid[LQ];
+};
+struct IvfItems {
+    std::vector<IvfItem> items;
+    std::vector<uint64_t> poff;
+    std::vector<uint32_t> plist;
+};
+IvfItems ivf_group_items(const vdb_ivf* ivf, const uint64_t* h_probes, uint32_t nq, uint32_t nprobe, uint32_t group,
+                         uint32_t tile, uint32_t min_range);
+// per-query merge of the items' partial lists ([items][group][K] keys) into d_keys [nq][K]
+void ivf_merge_items(const uint64_t* d_partial, const IvfItems& it, uint32_t nq, uint32_t K, uint64_t* d_keys, cudaStream_t st);
+// ivf_pq.cu: IndexPQ::knn_pq restricted to the probed lists. Candidate stage: the max(ef, k) = kk best (ADC, global id)
+// keys per query over the rows of the n_probes nearest lists, [nq][kk], KEY_NONE padded; then the exact rerank.
+void ivf_pq_adc_keys(const vdb_dataset* ds, const vdb_ivf* ivf, const vdb_pq* pq, const void* d_queries, uint32_t nq,
+                     uint32_t kk, uint32_t n_probes, uint64_t* d_keys, cudaStream_t st);
+void ivf_pq_knn_keys(const vdb_dataset* ds, const vdb_ivf* ivf, const vdb_pq* pq, const void* d_queries, uint32_t nq,
+                     uint32_t k, uint32_t ef, uint32_t n_probes, uint64_t* d_keys, cudaStream_t st);
 
 // rebuilds (distance, id) keys: key[j] = valid[j] ? make_key(dist[j], id[j]) : KEY_NONE
 void rekey(const float* d_dist, const uint32_t* d_ids, const uint8_t* d_valid, uint64_t count, uint64_t* d_keys,

@@ -164,15 +164,7 @@ __global__ void __launch_bounds__(IVF_THREADS) ivf_scan_kernel(const IvfScanPara
 // it, row range): the item's rows are streamed ONCE for all its queries (the K1 inner loop with gathered row ids), so
 // the HBM traffic drops from sum_q(rows visited by q) to sum_lists(ceil(Q_list / 8) * list rows). Every item writes a
 // k-best list per query slot; a per-query index of those partial lists drives the final merge.
-constexpr int LQ = 8;   // queries per item
-constexpr int LR = 4;   // rows per warp step
-
-struct IvfItem {
-    uint64_t row_begin;   // offset into members[]
-    uint32_t nrows;
-    uint32_t nq_valid;
-    uint32_t qid[LQ];
-};
+constexpr int LR = 4;   // rows per warp step (an item holds up to LQ queries, index.cuh)
 
 struct IvfListParams {
     const uint8_t* rows;
@@ -497,9 +489,9 @@ void ivf_destroy(vdb_ivf* ivf) {
     delete ivf;
 }
 
-static void ivf_list_major(const vdb_dataset* ds, const vdb_ivf* ivf, const QueryTile& qt, const uint64_t* probes,
-                           const std::vector<uint64_t>& off, uint32_t nq, uint32_t nprobe, uint32_t k, uint64_t* d_keys,
-                           cudaStream_t st) {
+IvfItems ivf_group_items(const vdb_ivf* ivf, const uint64_t* probes, uint32_t nq, uint32_t nprobe, uint32_t group,
+                         uint32_t tile, uint32_t min_range) {
+    const std::vector<uint64_t>& off = ivf->h_off;
     std::vector<std::vector<uint32_t>> by_list(ivf->nlist);
     for (uint32_t q = 0; q < nq; ++q)
         for (uint32_t j = 0; j < nprobe; ++j) {
@@ -508,17 +500,18 @@ static void ivf_list_major(const vdb_dataset* ds, const vdb_ivf* ivf, const Quer
         }
     // row-range size: enough items to fill the GPU a few times, rows per item a multiple of the warp tile
     uint64_t work = 0;  // sum over (list, query group) of rows
-    for (uint32_t l = 0; l < ivf->nlist; ++l) work += ceil_div<uint64_t>(by_list[l].size(), LQ) * (off[l + 1] - off[l]);
+    for (uint32_t l = 0; l < ivf->nlist; ++l) work += ceil_div<uint64_t>(by_list[l].size(), group) * (off[l + 1] - off[l]);
     const uint64_t target_items = (uint64_t)sm_count() * 16;
-    uint32_t range = (uint32_t)std::max<uint64_t>(IVF_WARPS * LR * 4, round_up<uint64_t>(ceil_div<uint64_t>(work, target_items), IVF_WARPS * LR));
-    std::vector<IvfItem> items;
+    uint32_t range = (uint32_t)std::max<uint64_t>(min_range, round_up<uint64_t>(ceil_div<uint64_t>(work, target_items), tile));
+    IvfItems out;
+    std::vector<IvfItem>& items = out.items;
     std::vector<std::vector<uint32_t>> qlists(nq);  // partial-list indices per query
     for (uint32_t l = 0; l < ivf->nlist; ++l) {
         const uint64_t len = off[l + 1] - off[l];
         if (len == 0) continue;
         const auto& qv = by_list[l];
-        for (size_t c = 0; c < qv.size(); c += LQ) {
-            const uint32_t nv = (uint32_t)std::min<size_t>(LQ, qv.size() - c);
+        for (size_t c = 0; c < qv.size(); c += group) {
+            const uint32_t nv = (uint32_t)std::min<size_t>(group, qv.size() - c);
             for (uint64_t r0 = 0; r0 < len; r0 += range) {
                 IvfItem it{};
                 it.row_begin = off[l] + r0;
@@ -526,25 +519,43 @@ static void ivf_list_major(const vdb_dataset* ds, const vdb_ivf* ivf, const Quer
                 it.nq_valid = nv;
                 for (uint32_t s = 0; s < nv; ++s) {
                     it.qid[s] = qv[c + s];
-                    qlists[qv[c + s]].push_back((uint32_t)(items.size() * LQ + s));
+                    qlists[qv[c + s]].push_back((uint32_t)(items.size() * group + s));
                 }
                 items.push_back(it);
             }
         }
     }
-    std::vector<uint64_t> poff(nq + 1, 0);
-    for (uint32_t q = 0; q < nq; ++q) poff[q + 1] = poff[q] + qlists[q].size();
-    std::vector<uint32_t> plist(poff[nq]);
-    for (uint32_t q = 0; q < nq; ++q) std::copy(qlists[q].begin(), qlists[q].end(), plist.begin() + poff[q]);
+    out.poff.assign(nq + 1, 0);
+    for (uint32_t q = 0; q < nq; ++q) out.poff[q + 1] = out.poff[q] + qlists[q].size();
+    out.plist.resize(out.poff[nq]);
+    for (uint32_t q = 0; q < nq; ++q) std::copy(qlists[q].begin(), qlists[q].end(), out.plist.begin() + out.poff[q]);
+    return out;
+}
+
+void ivf_merge_items(const uint64_t* d_partial, const IvfItems& it, uint32_t nq, uint32_t K, uint64_t* d_keys, cudaStream_t st) {
+    DevBuf d_poff(it.poff.size() * 8, st), d_plist(std::max<size_t>(4, it.plist.size() * 4), st);
+    VDB_CUDA(cudaMemcpyAsync(d_poff.p, it.poff.data(), it.poff.size() * 8, cudaMemcpyHostToDevice, st));
+    if (!it.plist.empty()) VDB_CUDA(cudaMemcpyAsync(d_plist.p, it.plist.data(), it.plist.size() * 4, cudaMemcpyHostToDevice, st));
+    const uint32_t PM = topk_segment_size(K, 256);
+    const size_t smem_m = TopkSmem::bytes(1, PM);
+    VDB_REQUIRE(smem_m <= 200 * 1024, "IVF merge: k=%u too large", K);
+    if (smem_m > 48 * 1024)
+        VDB_CUDA(cudaFuncSetAttribute(ivf_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m));
+    ivf_merge_kernel<<<nq, 256, smem_m, st>>>(d_partial, d_poff.as<uint64_t>(), d_plist.as<uint32_t>(), K, PM, PM - K - 256,
+                                              d_keys);
+    VDB_LAUNCHED();
+}
+
+static void ivf_list_major(const vdb_dataset* ds, const vdb_ivf* ivf, const QueryTile& qt, const uint64_t* probes,
+                           uint32_t nq, uint32_t nprobe, uint32_t k, uint64_t* d_keys, cudaStream_t st) {
+    const IvfItems grouped = ivf_group_items(ivf, probes, nq, nprobe, LQ, IVF_WARPS * LR, IVF_WARPS * LR * 4);
+    const std::vector<IvfItem>& items = grouped.items;
     if (items.empty()) {
         VDB_CUDA(cudaMemsetAsync(d_keys, 0xff, (size_t)nq * k * 8, st));
         return;
     }
-    DevBuf d_items(items.size() * sizeof(IvfItem), st), d_poff(poff.size() * 8, st), d_plist(std::max<size_t>(4, plist.size() * 4), st),
-        partial(items.size() * LQ * (size_t)k * 8, st);
+    DevBuf d_items(items.size() * sizeof(IvfItem), st), partial(items.size() * LQ * (size_t)k * 8, st);
     VDB_CUDA(cudaMemcpyAsync(d_items.p, items.data(), items.size() * sizeof(IvfItem), cudaMemcpyHostToDevice, st));
-    VDB_CUDA(cudaMemcpyAsync(d_poff.p, poff.data(), poff.size() * 8, cudaMemcpyHostToDevice, st));
-    if (!plist.empty()) VDB_CUDA(cudaMemcpyAsync(d_plist.p, plist.data(), plist.size() * 4, cudaMemcpyHostToDevice, st));
     const uint32_t period = 64;
     const uint32_t P = topk_segment_size(k, period);
     const size_t smem = (size_t)LQ * qt.qstride * 4 + TopkSmem::bytes(LQ, P);
@@ -579,14 +590,7 @@ static void ivf_list_major(const vdb_dataset* ds, const vdb_ivf* ivf, const Quer
         if (ds->metric == VDB_L2SQR) go(ivf_list_scan_kernel<VDB_L2SQR, 4>);
         else go(ivf_list_scan_kernel<VDB_COSINE, 4>);
     }
-    const uint32_t PM = topk_segment_size(k, 256);
-    const size_t smem_m = TopkSmem::bytes(1, PM);
-    VDB_REQUIRE(smem_m <= 200 * 1024, "IVF merge: k=%u too large", k);
-    if (smem_m > 48 * 1024)
-        VDB_CUDA(cudaFuncSetAttribute(ivf_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m));
-    ivf_merge_kernel<<<nq, 256, smem_m, st>>>(partial.as<uint64_t>(), d_poff.as<uint64_t>(), d_plist.as<uint32_t>(), k, PM,
-                                              PM - k - 256, d_keys);
-    VDB_LAUNCHED();
+    ivf_merge_items(partial.as<uint64_t>(), grouped, nq, k, d_keys, st);
 }
 
 __global__ void gather_bytes_rows_kernel(const uint8_t* __restrict__ src, uint32_t row_bytes, const uint32_t* __restrict__ idx,
@@ -613,7 +617,21 @@ void ivf_list_major_subset(const vdb_dataset* ds, const vdb_ivf* ivf, const void
     VDB_CUDA(cudaMemcpyAsync(h_probes.data(), pr.p, h_probes.size() * 8, cudaMemcpyDeviceToHost, st));
     VDB_CUDA(cudaStreamSynchronize(st));
     QueryTile qt = prepare_queries(ds, q.p, nsel, st);
-    ivf_list_major(ds, ivf, qt, h_probes.data(), ivf->h_off, nsel, nprobe, k, d_keys_sel, st);
+    ivf_list_major(ds, ivf, qt, h_probes.data(), nsel, nprobe, k, d_keys_sel, st);
+}
+
+DevBuf ivf_probe_keys(const vdb_dataset* ds, const vdb_ivf* ivf, const void* d_queries, uint32_t nq, uint32_t nprobe,
+                      cudaStream_t st) {
+    // exact query-centroid distances, probe order = find_n_nearest (k_means.rs:174-191)
+    DevBuf cdist((size_t)nq * ivf->nlist * 4, st), ckeys((size_t)nq * ivf->nlist * 8, st), probes((size_t)nq * nprobe * 8, st);
+    probe_distances(ds, ivf, d_queries, nq, cdist.as<float>(), st);
+    const uint64_t cnt = (uint64_t)nq * ivf->nlist;
+    probe_keys_kernel<<<(uint32_t)std::min<uint64_t>(ceil_div<uint64_t>(cnt, 256), 4096), 256, 0, st>>>(
+        cdist.as<float>(), cnt, ivf->nlist, ckeys.as<uint64_t>());
+    VDB_LAUNCHED();
+    launch_merge_keys(ckeys.as<uint64_t>(), 1, nq, ivf->nlist, false, nprobe, probes.as<uint64_t>(), nullptr, nullptr,
+                      nullptr, st);
+    return probes;
 }
 
 void ivf_knn_keys(const vdb_dataset* ds, const vdb_ivf* ivf, const void* d_queries, uint32_t nq, uint32_t k,
@@ -630,15 +648,8 @@ void ivf_knn_keys(const vdb_dataset* ds, const vdb_ivf* ivf, const void* d_queri
         return;
     }
     const uint32_t nprobe = std::min(n_probes, ivf->nlist);
-    // 1. exact query-centroid distances, probe order = find_n_nearest (k_means.rs:174-191)
-    DevBuf cdist((size_t)nq * ivf->nlist * 4, st), ckeys((size_t)nq * ivf->nlist * 8, st), probes((size_t)nq * nprobe * 8, st);
-    probe_distances(ds, ivf, d_queries, nq, cdist.as<float>(), st);
-    const uint64_t cnt = (uint64_t)nq * ivf->nlist;
-    probe_keys_kernel<<<(uint32_t)std::min<uint64_t>(ceil_div<uint64_t>(cnt, 256), 4096), 256, 0, st>>>(
-        cdist.as<float>(), cnt, ivf->nlist, ckeys.as<uint64_t>());
-    VDB_LAUNCHED();
-    launch_merge_keys(ckeys.as<uint64_t>(), 1, nq, ivf->nlist, false, nprobe, probes.as<uint64_t>(), nullptr, nullptr,
-                      nullptr, st);
+    // 1. probe order
+    DevBuf probes = ivf_probe_keys(ds, ivf, d_queries, nq, nprobe, st);
     // 2. list scan
     if (nq >= 4) {
         // probe table to the host (nq * nprobe keys): the grouping by list is host work, the item tables go back
@@ -651,7 +662,7 @@ void ivf_knn_keys(const vdb_dataset* ds, const vdb_ivf* ivf, const void* d_queri
             ivf_tensor_keys(ds, ivf, d_queries, probes.as<uint64_t>(), h_probes, nq, nprobe, k, d_keys, st))
             return;
         QueryTile qt = prepare_queries(ds, d_queries, nq, st);
-        ivf_list_major(ds, ivf, qt, h_probes, ivf->h_off, nq, nprobe, k, d_keys, st);
+        ivf_list_major(ds, ivf, qt, h_probes, nq, nprobe, k, d_keys, st);
         return;
     }
     QueryTile qt = prepare_queries(ds, d_queries, nq, st);

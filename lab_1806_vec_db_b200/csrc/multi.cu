@@ -890,19 +890,18 @@ vdb_pq* sharded_pq_create(const vdb_dataset* md, const void* h_codebooks, uint32
     return pq;
 }
 
-// IndexPQ::knn_pq for FlatIndex on the sharded set, identical to the unsharded call: (1) every shard's max(ef, k) best
-// codes by (ADC, global id) go to the queries' owners, (2) the owners merge them into the GLOBAL top-max(ef, k) and
-// peer-store their slice of it into every shard, (3) every shard reranks exactly the candidates it owns, (4) the [nq, k]
-// keys are merged on the owners.
-void sharded_pq_knn(const vdb_dataset* md, const vdb_pq* pq, const void* queries, uint32_t nq, uint32_t k, uint32_t ef,
-                    uint64_t* ids, float* dist, uint32_t* counts) {
+// IndexPQ::knn_pq on the sharded set (Flat, or IVF restricted to the probed lists), identical to the unsharded call:
+// (1) every shard's max(ef, k) best codes by (ADC, global id) - `candidates` - go to the queries' owners, (2) the owners
+// merge them into the GLOBAL top-max(ef, k) and peer-store their slice of it into every shard, (3) every shard reranks
+// exactly the candidates it owns, (4) the [nq, k] keys are merged on the owners.
+static void sharded_knn_pq(const vdb_dataset* md, const void* queries, uint32_t nq, uint32_t k, uint32_t ef, uint64_t* ids,
+                           float* dist, uint32_t* counts, const KeyProducer& candidates) {
     vdb_sharded_state* S = md->sharded;
     if (nq == 0) return;
     if (k == 0) {
         memset(counts, 0, (size_t)nq * 4);
         return;
     }
-    VDB_REQUIRE(pq->shards.size() == S->shards.size(), "PQ table was not built on this sharded set");
     VDB_REQUIRE(nq <= SHARD_QUERY_CHUNK, "sharded knn_pq: at most %u queries per call", SHARD_QUERY_CHUNK);
     std::lock_guard<std::mutex> lk(S->call_mu);
     const uint32_t G = (uint32_t)S->shards.size(), kk = std::max(ef, k);
@@ -936,7 +935,7 @@ void sharded_pq_knn(const vdb_dataset* md, const vdb_pq* pq, const void* queries
         Shard& sh = S->shards[s];
         VDB_CUDA(cudaMemcpyAsync(sh.q_all.p, queries, (size_t)nq * rb, cudaMemcpyHostToDevice, sh.st));
         keys[s] = DevBuf((size_t)nq * kk * 8, sh.st);
-        pq_adc_keys(sh.ds, pq->shards[s], sh.q_all.p, nq, kk, keys[s].as<uint64_t>(), sh.st);
+        candidates(s, sh.q_all.p, nq, kk, keys[s].as<uint64_t>(), sh.st);
         PtrList dk{}, df{};
         for (uint32_t h = 0; h < G; ++h) {
             uint32_t lo, hi;
@@ -997,6 +996,30 @@ void sharded_pq_knn(const vdb_dataset* md, const vdb_pq* pq, const void* queries
         VDB_CUDA(cudaStreamSynchronize(sh.st));
     });
     run_job(S, ph);
+}
+
+void sharded_pq_knn(const vdb_dataset* md, const vdb_pq* pq, const void* queries, uint32_t nq, uint32_t k, uint32_t ef,
+                    uint64_t* ids, float* dist, uint32_t* counts) {
+    vdb_sharded_state* S = md->sharded;
+    VDB_REQUIRE(nq == 0 || k == 0 || pq->shards.size() == S->shards.size(), "PQ table was not built on this sharded set");
+    sharded_knn_pq(md, queries, nq, k, ef, ids, dist, counts,
+                   [&](uint32_t s, const void* d_q, uint32_t n, uint32_t kk, uint64_t* d_keys, cudaStream_t st) {
+                       pq_adc_keys(S->shards[s].ds, pq->shards[s], d_q, n, kk, d_keys, st);
+                   });
+}
+
+void sharded_ivf_knn_pq(const vdb_dataset* md, const vdb_ivf* ivf, const vdb_pq* pq, const void* queries, uint32_t nq, uint32_t k,
+                        uint32_t ef, uint32_t n_probes, uint64_t* ids, float* dist, uint32_t* counts) {
+    vdb_sharded_state* S = md->sharded;
+    VDB_REQUIRE(ivf->shards.size() == S->shards.size() && ivf->parent == md && ivf->n == md->n,
+                "IVF index was built for a different vector set");
+    VDB_REQUIRE(pq->shards.size() == S->shards.size() && pq->n == md->n,
+                "PQ table was built for a different vector set (it must be rebuilt after add/delete)");
+    VDB_REQUIRE(n_probes > 0, "The number of probes should be greater than 0.");
+    sharded_knn_pq(md, queries, nq, k, ef, ids, dist, counts,
+                   [&](uint32_t s, const void* d_q, uint32_t n, uint32_t kk, uint64_t* d_keys, cudaStream_t st) {
+                       ivf_pq_adc_keys(S->shards[s].ds, ivf->shards[s], pq->shards[s], d_q, n, kk, n_probes, d_keys, st);
+                   });
 }
 
 uint32_t sharded_count(const vdb_dataset* md) { return md->sharded ? (uint32_t)md->sharded->shards.size() : 0; }

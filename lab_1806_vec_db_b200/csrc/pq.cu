@@ -19,6 +19,7 @@
 #include <cstdlib>
 #include <cstring>
 
+#include "adc.cuh"
 #include "index.cuh"
 #include "topk.cuh"
 
@@ -290,7 +291,6 @@ __global__ void pq_lut_kernel(const T* __restrict__ q, uint32_t nq, uint32_t dim
 }
 
 // ---- K8: ADC scan ----------------------------------------------------------------------------------
-constexpr int ADC_THREADS = 512;
 
 struct AdcParams {
     const uint32_t* codes_t;
@@ -337,21 +337,6 @@ __global__ void __launch_bounds__(ADC_THREADS) pq_adc_scan_kernel(AdcParams p) {
     float qn[NQ];
 #pragma unroll
     for (int q = 0; q < NQ; ++q) qn[q] = (METRIC == VDB_COSINE && q < (int)nq_valid) ? p.qcache[q] : 0.f;
-    constexpr int KC = NBITS == 4 ? 16 : 256;
-
-    // one table lookup for all NQ queries; the branch on LUT_SMEM is compile-time so the shared-memory path
-    // compiles to LDS (32-bit shared addressing), never to generic loads
-    auto lookup = [&](uint32_t e, float (&sum)[NQ], float& cdp) {
-        if constexpr (LUT_SMEM) {
-#pragma unroll
-            for (int q = 0; q < NQ; ++q) sum[q] = __fadd_rn(sum[q], s_lut[q * tab + e]);
-            if (METRIC == VDB_COSINE) cdp = __fadd_rn(cdp, s_dc[e]);
-        } else {
-#pragma unroll
-            for (int q = 0; q < NQ; ++q) sum[q] = __fadd_rn(sum[q], __ldg(p.lut + (size_t)q * tab + e));
-            if (METRIC == VDB_COSINE) cdp = __fadd_rn(cdp, __ldg(p.dist_cache + e));
-        }
-    };
 
     for (uint32_t it = 0; it < p.iters; ++it) {
         const uint64_t tile = (uint64_t)it * gridDim.x + blockIdx.x;
@@ -362,44 +347,9 @@ __global__ void __launch_bounds__(ADC_THREADS) pq_adc_scan_kernel(AdcParams p) {
 #pragma unroll
         for (int q = 0; q < NQ; ++q) sum[q] = 0.f;
         const bool in = row < p.n;
-        if (in) {
-            const uint32_t* cw = p.codes_t + blk * p.words * 32 + lane;
-            uint32_t g = 0;
-            uint32_t next = cw[0];
-            for (uint32_t w = 0; w < p.words; ++w) {
-                const uint32_t word = next;
-                if (w + 1 < p.words) next = cw[(size_t)(w + 1) * 32];  // prefetch the next code word
-                if (NBITS == 4) {
-                    if (LUT_SMEM && METRIC == VDB_L2SQR && g + 8 <= p.m) {
-                        // full word: issue all 8 x NQ table reads first, then add in the reference's group order
-                        float v[8][NQ];
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            const uint32_t e = (g + i) * KC + ((word >> (4 * i)) & 0xfu);
-#pragma unroll
-                            for (int q = 0; q < NQ; ++q) v[i][q] = s_lut[q * tab + e];
-                        }
-#pragma unroll
-                        for (int i = 0; i < 8; ++i)
-#pragma unroll
-                            for (int q = 0; q < NQ; ++q) sum[q] = __fadd_rn(sum[q], v[i][q]);
-                    } else if (g + 8 <= p.m) {  // full word: 8 groups, no per-nibble bound checks
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) lookup((g + i) * KC + ((word >> (4 * i)) & 0xfu), sum, cdp);
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < 8; ++i)
-                            if (g + i < p.m) lookup((g + i) * KC + ((word >> (4 * i)) & 0xfu), sum, cdp);
-                    }
-                    g += 8;
-                } else {
-#pragma unroll
-                    for (int i = 0; i < 4; ++i)
-                        if (g + i < p.m) lookup((g + i) * KC + ((word >> (8 * i)) & 0xffu), sum, cdp);
-                    g += 4;
-                }
-            }
-        }
+        if (in)
+            adc_row_sum<NQ, NBITS, METRIC, LUT_SMEM>(p.codes_t + blk * p.words * 32 + lane, p.words, p.m, tab,
+                                                     LUT_SMEM ? s_lut : p.lut, LUT_SMEM ? s_dc : p.dist_cache, sum, cdp);
         bool want = false;
 #pragma unroll
         for (int q = 0; q < NQ; ++q) {
@@ -610,8 +560,6 @@ __global__ void scatter_u64_rows_kernel(const uint64_t* __restrict__ src, uint32
     for (uint32_t e = threadIdx.x; e < width; e += blockDim.x) dst[(size_t)idx[i] * width + e] = src[(size_t)i * width + e];
 }
 
-constexpr size_t ADC_SMEM_MAX = 200 * 1024;
-
 template <int NQ>
 static void adc_launch(const vdb_pq* pq, const AdcParams& p, bool lut_smem, uint32_t grid, uint32_t groups, size_t smem,
                        cudaStream_t st) {
@@ -655,11 +603,8 @@ static void adc_scan(const vdb_pq* pq, const float* d_lut, const float* d_qcache
         return s;
     };
     static const int nqt_env = getenv("VDB_ADC_NQ") ? atoi(getenv("VDB_ADC_NQ")) : 0;
-    int nqt = (nqt_env == 1 || nqt_env == 2 || nqt_env == 4) ? nqt_env : 4;
     bool lut_smem = true;
-    while (nqt > 1 && (uint32_t)(nqt >> 1) >= nq) nqt >>= 1;  // no wider than the batch
-    while (nqt > 1 && smem_for(nqt, true) > ADC_SMEM_MAX) nqt >>= 1;
-    if (smem_for(nqt, true) > ADC_SMEM_MAX) lut_smem = false;
+    const int nqt = adc_queries_per_cta((nqt_env == 1 || nqt_env == 2 || nqt_env == 4) ? nqt_env : 4, nq, smem_for, &lut_smem);
     VDB_REQUIRE(smem_for(nqt, lut_smem) <= ADC_SMEM_MAX, "ADC scan: ef=%u too large for the fused top-k", K);
     const uint64_t tiles = ceil_div<uint64_t>(pq->n, ADC_THREADS);
     // one wave: resident CTAs per SM is limited by shared memory (LUTs + top-k segments)
@@ -863,6 +808,8 @@ __global__ void pq_sample_codes_kernel(const uint8_t* __restrict__ codes, uint64
 }
 
 // ---- table construction -------------------------------------------------------------------------------
+static std::atomic<uint64_t> g_pq_serial{0};
+
 vdb_pq* pq_create(const vdb_dataset* ds, const void* h_codebooks, uint32_t m, uint32_t n_bits,
                   const uint8_t* h_codes_in, uint8_t* h_codes_out) {
     VDB_REQUIRE(n_bits == 4 || n_bits == 8, "n_bits must be 4 or 8 in PQTable.");
@@ -871,6 +818,7 @@ vdb_pq* pq_create(const vdb_dataset* ds, const void* h_codebooks, uint32_t m, ui
     cudaStream_t st = nullptr;
     try {
         pq->device = ds->device;
+        pq->serial = ++g_pq_serial;
         pq->dim = ds->dim;
         pq->m = m;
         pq->n_bits = n_bits;

@@ -563,6 +563,31 @@ class IVFIndex:
     def knn(self, query, k):
         return self.knn_with_ef(query, k, self.default_n_probes)
 
+    def knn_pq_batch(self, queries, k, ef, pq_table, n_probes=None):
+        """IndexPQ::knn_pq restricted to the n_probes nearest lists (default: default_n_probes): the max(ef, k) best
+        codes by (ADC, id) over the rows of those lists, re-scored exactly, the k best kept. With n_probes >= nlist
+        this is FlatIndex.knn_pq_batch. Returns (ids [nq,k] u64, dist [nq,k] f32, counts [nq] u32)."""
+        vs = self.vec_set
+        q = _as_rows(queries, vs.dtype)
+        if q.shape[1] != vs.dim:
+            raise ValueError("The dimension of the query doesn't match.")
+        if L.metric_code(pq_table.config.dist) != vs.metric:
+            raise ValueError("Distance algorithm mismatch.")
+        n_probes = self.default_n_probes if n_probes is None else n_probes
+        if n_probes <= 0:
+            raise ValueError("The number of probes should be greater than 0.")
+        nq = q.shape[0]
+        ids = np.full((nq, k), np.iinfo(np.uint64).max, np.uint64)
+        dist = np.full((nq, k), np.nan, np.float32)
+        counts = np.zeros(nq, np.uint32)
+        L.check(L.lib().vdb_ivf_knn_pq(vs._h, self._h, pq_table._h, L.ptr(q), nq, k, ef, n_probes, L.ptr(ids), L.ptr(dist),
+                                       L.ptr(counts)))
+        return ids, dist, counts
+
+    def knn_pq(self, query, k, ef, pq_table):
+        """IndexPQ::knn_pq with the index's default probe count (ivf_index.rs:97, set_default_ef)."""
+        return _pairs(*self.knn_pq_batch(np.asarray(query).reshape(1, -1), k, ef, pq_table))[0]
+
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
             L.lib().vdb_ivf_destroy(self._h)

@@ -6,7 +6,7 @@
 //! A maintainer adds this file as `src/gpu.rs` (it uses `pub(crate)` fields of `HNSWIndex`, so it lives inside the
 //! crate), links `libvdb_b200.so` from build.rs (`println!("cargo:rustc-link-lib=dylib=vdb_b200")`) and swaps
 //!   FlatIndex<T>  -> GpuFlatIndex<T>      (IndexKNN, IndexPQ, IndexFromVecSet;   src/index_algorithm/flat_index.rs)
-//!   IVFIndex<T>   -> GpuIvfIndex<T>       (IndexKNN, IndexKNNWithEf, IndexFromVecSet; src/index_algorithm/ivf_index.rs)
+//!   IVFIndex<T>   -> GpuIvfIndex<T>       (IndexKNN, IndexKNNWithEf, IndexPQ, IndexFromVecSet; ivf_index.rs)
 //!   HNSWIndex<T>  -> GpuHnswIndex<T>      (IndexKNN, IndexKNNWithEf, IndexPQ, build_on_vec_set; hnsw_index.rs)
 //!   KMeans::from_vec_set / find_nearest   -> gpu_kmeans_from_vec_set / gpu_find_nearest_batch (src/distance/k_means.rs)
 //!   PQTable::from_vec_set                 -> gpu_pq_table_from_vec_set            (src/distance/pq_table.rs:141-191)
@@ -71,6 +71,8 @@ extern "C" {
     pub fn vdb_ivf_destroy(ivf: *mut vdb_ivf) -> c_int;
     pub fn vdb_ivf_knn(ds: *const vdb_dataset, ivf: *const vdb_ivf, queries: *const c_void, nq: u32, k: u32,
                        n_probes: u32, ids: *mut u64, dist: *mut f32, counts: *mut u32) -> c_int;
+    pub fn vdb_ivf_knn_pq(ds: *const vdb_dataset, ivf: *const vdb_ivf, pq: *const vdb_pq, queries: *const c_void, nq: u32,
+                          k: u32, ef: u32, n_probes: u32, ids: *mut u64, dist: *mut f32, counts: *mut u32) -> c_int;
     pub fn vdb_hnsw_build(ds: *const vdb_dataset, m: u32, ef_construction: u32, levels: *const u32, max_batch: u32,
                           out: *mut *mut vdb_hnsw) -> c_int;
     pub fn vdb_hnsw_destroy(h: *mut vdb_hnsw) -> c_int;
@@ -282,6 +284,7 @@ pub struct GpuIvfIndex<T: Scalar> {
     pub inner: IVFIndex<T>,
     ds: Mirror,
     ivf: *mut vdb_ivf,
+    pq: Mutex<Option<PqMirror>>,
 }
 unsafe impl<T: Scalar> Send for GpuIvfIndex<T> {}
 unsafe impl<T: Scalar> Sync for GpuIvfIndex<T> {}
@@ -310,7 +313,7 @@ impl<T: Scalar> IndexFromVecSet<T> for GpuIvfIndex<T> {
         check(unsafe { vdb_ivf_create(ds.0, rows_ptr(&k_means.centroids), k as u32, assign.as_mut_ptr(), &mut ivf) });
         let mut clusters = vec![vec![]; k];
         for (i, &c) in assign.iter().enumerate() { clusters[c as usize].push(i); }
-        Self { inner: IVFIndex { dist, default_n_probes: 4, vec_set, config, clusters, k_means }, ds, ivf }
+        Self { inner: IVFIndex { dist, default_n_probes: 4, vec_set, config, clusters, k_means }, ds, ivf, pq: Mutex::new(None) }
     }
 }
 impl<T: Scalar> IndexKNN<T> for GpuIvfIndex<T> {
@@ -323,6 +326,20 @@ impl<T: Scalar> IndexKNNWithEf<T> for GpuIvfIndex<T> {
         let (mut ids, mut dist, mut cnt) = (vec![0u64; k], vec![0f32; k], vec![0u32; 1]);
         check(unsafe { vdb_ivf_knn(self.ds.0, self.ivf, query.as_ptr() as _, 1, k as u32, n_probes as u32,
                                    ids.as_mut_ptr(), dist.as_mut_ptr(), cnt.as_mut_ptr()) });
+        pairs(&ids, &dist, cnt[0])
+    }
+}
+
+impl<T: Scalar> IndexPQ<T> for GpuIvfIndex<T> {
+    /// IVF knn_pq (the reference has none; INTEGRATION.md defines it): FlatIndex::knn_pq (flat_index.rs:84-104)
+    /// restricted to the rows of the default_n_probes nearest lists
+    fn knn_pq(&self, query: &[T], k: usize, ef: usize, pq_table: &PQTable<T>) -> Vec<CandidatePair> {
+        assert_eq!(self.inner.dist, pq_table.config.dist, "Distance algorithm mismatch.");
+        let pq = pq_mirror(&self.pq, self.ds.0, pq_table);
+        let (mut ids, mut dist, mut cnt) = (vec![0u64; k], vec![0f32; k], vec![0u32; 1]);
+        check(unsafe { vdb_ivf_knn_pq(self.ds.0, self.ivf, pq, query.as_ptr() as _, 1, k as u32, ef as u32,
+                                      self.inner.default_n_probes as u32, ids.as_mut_ptr(), dist.as_mut_ptr(),
+                                      cnt.as_mut_ptr()) });
         pairs(&ids, &dist, cnt[0])
     }
 }
