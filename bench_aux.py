@@ -6,6 +6,11 @@
   C4  PQ   m=240, 4 bits, k-means on 10k rows (20 iters), Flat+PQ scan, ef in {240..600 step 60}, k=10
            (config/bench_pq_240_hnsw.toml:16-23, examples/bench.rs protocol: recall@10 vs Flat ground truth)
 
+  hnsw   C5 HNSW M=16, ef_construction=200, ef in {120..360 step 40}, k=10 (config/bench_hnsw.toml). With --gpus 1,2,4,8:
+           the same index on a row-sharded set of G GPUs (one replica of rows + graph per GPU, every search one call whose
+           batch is split over the replicas): build time, replication time, QPS at 1000 and 10000 queries over the ef
+           sweep, recall, and whether the ids equal the 1-GPU run's
+
   ivfpq  IVF + PQ (IVFIndex.knn_pq): the C3 lists and the C4 table, nprobe in {8,16,32} x ef in {60,120,240}, at nq =
            1000 and nq = 1, next to IVF knn_with_ef and Flat knn_pq at the same settings, with the ADC lookups of the
            scan and their floor (32 shared-memory reads per clock per SM)
@@ -63,6 +68,7 @@ def main():
     ap.add_argument("--pq-m", type=int, default=240)
     ap.add_argument("--ef", default="240:600:60", help="start:end:step of the PQ ef sweep")
     ap.add_argument("--data", choices=("synth", "clustered"), default="synth")
+    ap.add_argument("--gpus", default=None, help="hnsw: GPU counts to run the index on, e.g. 1,2,4,8 (host-pointer calls)")
     args = ap.parse_args()
     what = set(args.what.split(","))
     import torch
@@ -191,7 +197,9 @@ def main():
                               "achieved_code_gbs": gbs, "cpu_qps": cpu_qps, "cpu_cores": cores, "cpu_queries": nc,
                               "gpu_vs_oracle_exact_id_rate": same}), flush=True)
 
-    if "hnsw" in what:
+    if "hnsw" in what and args.gpus:
+        hnsw_gpus_sweep(args, V, L, lib, base_host, flat, gen, test1000, dev, k)
+    elif "hnsw" in what:
         # C5: config/bench_hnsw.toml (M = 16 default, ef_construction = 200, ef 120..360 step 40, k = 10)
         L.check(lib.vdb_prof_reset())
         L.check(lib.vdb_prof_enable(1))
@@ -266,6 +274,63 @@ def card_info():
     except (OSError, ValueError, IndexError, subprocess.SubprocessError):
         info["power_limit_w"] = info["max_sm_clock_mhz"] = None
     return info
+
+
+def hnsw_gpus_sweep(args, V, L, lib, base_host, flat, gen, test1000, dev, k):
+    """C5 on G = 1, 2, ... GPUs: init_devices(range(G)) row-shards the set, the HNSW index keeps one replica per GPU. Same
+    levels for every G; G = 1 is the unsharded index. Searches are host-pointer calls (vdb_hnsw_knn), timed end to end."""
+    import torch
+    card = card_info()
+    have = torch.cuda.device_count()
+    nqs = (1000, 10000)
+    q_all = gen(test1000, 0, max(nqs), 43, dev).cpu().numpy()
+    gt = flat.knn_batch(q_all, k)[0].astype(np.int64)
+    levels = V.hnsw_rand_levels(args.n, args.hnsw_m, np.random.default_rng(42))
+    cfg = V.HNSWConfig(0, args.hnsw_efc, args.hnsw_m)
+    e0, e1, es = (int(x) for x in args.hnsw_ef.split(":"))
+    ids_one = {}
+    for g in (int(x) for x in args.gpus.split(",")):
+        if g > have:
+            print(json.dumps({"config": "C5 HNSW multi-GPU", "gpus": g, "skipped": f"{have} GPU(s) visible", **card}), flush=True)
+            continue
+        V.init_devices(list(range(g)) if g > 1 else [])
+        vs = V.DeviceVecSet(base_host, "l2sqr")
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        hn = V.HNSWIndex(vs, cfg, levels=levels)
+        t_build = time.perf_counter() - t0
+        # replication alone: the built graph loaded onto the same set again (rows gathered onto every replica, the graph
+        # copied into each)
+        links0, len0 = hn.level0_links()
+        lv, ul, un = hn.upper_links()
+        ul, un = (ul, un) if un.size else (np.zeros(1, np.uint32), np.zeros(1, np.uint32))
+        ep, el = hn.enter_point
+        h2 = C.c_void_p()
+        t0 = time.perf_counter()
+        L.check(lib.vdb_hnsw_create_from_graph(vs._h, args.hnsw_m, args.hnsw_efc, L.ptr(lv), L.ptr(links0), L.ptr(len0), L.ptr(ul),
+                                               L.ptr(un), ep, el, C.byref(h2)))
+        t_rep = time.perf_counter() - t0
+        L.check(lib.vdb_hnsw_destroy(h2))
+        print(json.dumps({"config": "C5 HNSW multi-GPU build", "gpus": g, "n": args.n, "M": args.hnsw_m,
+                          "ef_construction": args.hnsw_efc, "build_s": t_build, "replicate_s": t_rep, **card}), flush=True)
+        for nq in nqs:
+            q = q_all[:nq]
+            for ef in range(e0, e1 + 1, es):
+                hn.knn_with_ef_batch(q, k, ef)
+                reps = 3
+                t0 = time.perf_counter()
+                for _ in range(reps):
+                    ids = hn.knn_with_ef_batch(q, k, ef)[0]
+                ms = (time.perf_counter() - t0) * 1e3 / reps
+                if g == 1:
+                    ids_one[(nq, ef)] = ids
+                one = ids_one.get((nq, ef))
+                print(json.dumps({"config": "C5 HNSW multi-GPU search", "gpus": g, "nq": nq, "ef": ef, "k": k,
+                                  "qps": nq / ms * 1e3, "ms_per_batch": ms, "recall@10": recall_at(ids.astype(np.int64), gt[:nq]),
+                                  "ids_equal_1gpu": None if one is None else bool((ids == one).all()), **card}), flush=True)
+        hn.close()
+        vs.close()
+    V.init_devices([])
 
 
 def ivfpq_sweep(args, V, L, O, lib, vs, flat, q_dev, q_host, base_host, gt_ids, st, dev_out, build_ivf, build_pq, k, cores):

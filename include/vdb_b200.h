@@ -328,6 +328,12 @@ int vdb_ivf_knn_keys_dev(const vdb_dataset* ds, const vdb_ivf* ivf, const void* 
                          uint32_t n_probes, uint64_t* d_keys, void* stream);
 
 /* ---- HNSW ------------------------------------------------------------------------------------- */
+/* Row-sharded `ds` (vdb_init with several devices): build / create_from_graph keep one replica of all rows and the whole
+ * graph per shard entry (built once, loaded into the others; ids stay id_base + row), and vdb_hnsw_knn / _knn_pq split
+ * the batch into min(G, nq) contiguous slices, one per replica, in one re-entrant call: results are bit-identical to the
+ * unsharded index. knn_pq takes a table created on the same sharded set. info / links0 / upper answer from replica 0,
+ * overflow / evals sum the replicas (evals resets all of them). vdb_hnsw_append and the `_dev` searches return
+ * VDB_EUNSUPPORTED there; an index or table of another set returns VDB_EINVAL. */
 /* HNSWIndex::build_on_vec_set (src/index_algorithm/hnsw_index.rs:585-600; IndexBuilder::new :495-537, add :538-572,
  * add_parallel :399-457) over the rows of `ds` in row order, graph resident on the device. M / ef_construction as in
  * HNSWConfig (:41-59; max_m0 = 2 M, ef_construction = max(ef_construction, 2 M)). levels[i] = rand_level (:145-149)

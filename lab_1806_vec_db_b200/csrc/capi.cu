@@ -182,6 +182,28 @@ void host_search(int device, const void* queries, uint32_t nq, size_t qbytes_per
 }
 }  // namespace
 
+namespace vdb {
+// an unsharded dataset over rows already on `device` (not owned: the caller frees them unless it sets `owned`)
+vdb_dataset* adopt_dataset_on(int device, const void* d_rows, uint64_t n, uint32_t dim, uint32_t pitch, int dtype, int metric,
+                              uint64_t id_base) {
+    VDB_REQUIRE(((uintptr_t)d_rows & 15) == 0, "device rows must be 16-byte aligned");
+    auto ds = new vdb_dataset();
+    ds->device = device;
+    ds->d_rows = const_cast<void*>(d_rows);
+    ds->owned = false;
+    ds->n = ds->cap = n;
+    ds->dim = dim;
+    ds->pitch = pitch;
+    ds->dtype = dtype;
+    ds->metric = metric;
+    ds->id_base = id_base;
+    return ds;
+}
+// the calling thread's stream on the current device (the stream of the host-pointer entry points)
+cudaStream_t thread_stream() { return CallStream().s; }
+}  // namespace vdb
+using vdb::adopt_dataset_on;
+
 struct vdb_batcher {
     std::mutex mu;
     std::condition_variable cv;
@@ -262,22 +284,6 @@ static vdb_dataset* upload_dataset_on(int device, const void* rows, uint64_t n, 
         delete ds;
         throw;
     }
-    return ds;
-}
-
-static vdb_dataset* adopt_dataset_on(int device, const void* d_rows, uint64_t n, uint32_t dim, uint32_t pitch, int dtype,
-                                     int metric, uint64_t id_base) {
-    VDB_REQUIRE(((uintptr_t)d_rows & 15) == 0, "device rows must be 16-byte aligned");
-    auto ds = new vdb_dataset();
-    ds->device = device;
-    ds->d_rows = const_cast<void*>(d_rows);
-    ds->owned = false;
-    ds->n = ds->cap = n;
-    ds->dim = dim;
-    ds->pitch = pitch;
-    ds->dtype = dtype;
-    ds->metric = metric;
-    ds->id_base = id_base;
     return ds;
 }
 

@@ -1040,7 +1040,8 @@ static void exact_topk_of(const vdb_dataset* ds, const vdb_hnsw* h, const void* 
 // re-evaluated by the pair kernel that also serves vdb_gather_dist
 void hnsw_knn_keys(const vdb_dataset* ds, const vdb_hnsw* h, const void* d_queries, uint32_t nq, uint32_t k, uint32_t ef_in,
                    uint64_t* d_keys, cudaStream_t st) {
-    VDB_REQUIRE(ds->n == h->n && ds->dim == h->dim && ds->dtype == h->dtype && ds->metric == h->metric,
+    // an index of a row-sharded set has no arrays of its own (its replicas do)
+    VDB_REQUIRE(!h->rep && ds->n == h->n && ds->dim == h->dim && ds->dtype == h->dtype && ds->metric == h->metric,
                 "HNSW index was built for a different vector set");
     if (nq == 0 || k == 0) return;
     if (h->n == 0) {
@@ -1082,10 +1083,10 @@ void hnsw_knn_keys(const vdb_dataset* ds, const vdb_hnsw* h, const void* d_queri
 // with the exact cached form and the k best by (distance, id) returned (ResultSet::pq_resort, candidate_pair.rs:102-108)
 void hnsw_knn_pq_keys(const vdb_dataset* ds, const vdb_hnsw* h, const vdb_pq* pq, const void* d_queries, uint32_t nq, uint32_t k,
                       uint32_t ef_in, uint64_t* d_keys, cudaStream_t st) {
-    VDB_REQUIRE(ds->n == h->n && ds->dim == h->dim && ds->dtype == h->dtype && ds->metric == h->metric,
+    VDB_REQUIRE(!h->rep && ds->n == h->n && ds->dim == h->dim && ds->dtype == h->dtype && ds->metric == h->metric,
                 "HNSW index was built for a different vector set");
     VDB_REQUIRE(pq->metric == ds->metric, "Distance algorithm mismatch.");
-    VDB_REQUIRE(pq->n == ds->n && pq->dim == ds->dim, "PQ table was built for a different vector set");
+    VDB_REQUIRE(pq->shards.empty() && pq->n == ds->n && pq->dim == ds->dim, "PQ table was built for a different vector set");
     VDB_REQUIRE(pq->n_bits == 4, "HNSW + PQ search supports 4-bit codes");
     if (nq == 0 || k == 0) return;
     if (h->n == 0) {

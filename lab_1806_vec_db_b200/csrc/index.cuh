@@ -1,5 +1,6 @@
 // index.cuh — device mirrors of PQTable / IVFIndex and the k-means / pair-distance launchers.
 #pragma once
+#include <atomic>
 #include <memory>
 #include <mutex>
 #include <vector>
@@ -32,6 +33,7 @@ struct vdb_pq {
     bool dec_ok = false;
     float dec_scale = 1.0f, dec_ex = 0.f;
     std::vector<vdb_pq*> shards;    // row-sharded parent (multi.cu): one table per shard, the arrays above stay empty
+    const struct vdb_dataset* parent = nullptr;   // the row-sharded set a parent table was built on
 };
 
 // device mirror of IVFIndex<T> (reference src/index_algorithm/ivf_index.rs:34-47)
@@ -69,6 +71,7 @@ struct vdb_ivf {
 };
 
 // device mirror of HNSWIndex<T> (reference src/index_algorithm/hnsw_index.rs:99-141)
+struct HnswReplicas;
 struct vdb_hnsw {
     int device = 0;
     uint64_t n = 0;
@@ -87,6 +90,22 @@ struct vdb_hnsw {
     uint32_t* d_overflow = nullptr;    // neighbours a search could not record in its visited set (must stay 0)
     int64_t enter_point = -1;
     int enter_level = -1;
+    // index of a row-sharded set (multi.cu): the scalars above are replica 0's, the arrays stay empty
+    HnswReplicas* rep = nullptr;
+};
+
+// HNSW on a row-sharded set: a graph walk needs every row, so each shard entry holds a full replica (all n rows and the
+// same graph) and a search splits its batch over the replicas
+struct HnswPqReplicas;   // one PQ table's codes over all rows, one vdb_pq per replica (multi.cu)
+struct HnswReplicas {
+    const struct vdb_dataset* parent = nullptr;   // the row-sharded set the index was built on
+    std::vector<vdb_dataset*> ds;                 // replica r: all n rows on shard r's device, ids id_base + row
+    std::vector<vdb_hnsw*> h;                     // replica r: the graph over ds[r]
+    std::atomic<uint32_t> next{0};                // first replica of the next call with fewer queries than replicas
+    std::mutex pq_mu;                             // guards `pq`
+    // built by the first knn_pq call with a table, rebuilt when a call brings another table; a call holds its own
+    // reference, so a rebuild never frees codes a running search reads
+    std::shared_ptr<const HnswPqReplicas> pq;
 };
 
 namespace vdb {
@@ -102,6 +121,16 @@ void sharded_pq_knn(const vdb_dataset* md, const vdb_pq* pq, const void* queries
                     uint64_t* ids, float* dist, uint32_t* counts);
 void sharded_ivf_knn_pq(const vdb_dataset* md, const vdb_ivf* ivf, const vdb_pq* pq, const void* queries, uint32_t nq, uint32_t k,
                         uint32_t ef, uint32_t n_probes, uint64_t* ids, float* dist, uint32_t* counts);
+// multi.cu: HNSW on a row-sharded dataset (one replica per shard entry)
+vdb_hnsw* sharded_hnsw_build(const vdb_dataset* md, uint32_t M, uint32_t ef_construction, const uint32_t* h_levels,
+                             uint32_t max_batch);
+vdb_hnsw* sharded_hnsw_from_graph(const vdb_dataset* md, uint32_t M, uint32_t ef_construction, const uint32_t* h_levels,
+                                  const uint32_t* links0, const uint32_t* len0, const uint32_t* ulinks, const uint32_t* ulen,
+                                  int64_t enter_point, int32_t enter_level);
+void sharded_hnsw_destroy(vdb_hnsw* h);
+// pq == nullptr: knn_with_ef, else knn_pq
+void sharded_hnsw_knn(const vdb_dataset* md, const vdb_hnsw* h, const vdb_pq* pq, const void* queries, uint32_t nq, uint32_t k,
+                      uint32_t ef, uint64_t* ids, float* dist, uint32_t* counts);
 
 // hnsw.cu
 vdb_hnsw* hnsw_build(const vdb_dataset* ds, uint32_t M, uint32_t ef_construction, const uint32_t* h_levels, uint32_t max_batch);

@@ -887,6 +887,8 @@ vdb_pq* sharded_pq_create(const vdb_dataset* md, const void* h_codebooks, uint32
         throw;
     }
     cudaSetDevice(prev);
+    pq->serial = pq->shards.front()->serial;   // unique: shard tables are never handed out on their own
+    pq->parent = md;
     return pq;
 }
 
@@ -1020,6 +1022,289 @@ void sharded_ivf_knn_pq(const vdb_dataset* md, const vdb_ivf* ivf, const vdb_pq*
                    [&](uint32_t s, const void* d_q, uint32_t n, uint32_t kk, uint64_t* d_keys, cudaStream_t st) {
                        ivf_pq_adc_keys(S->shards[s].ds, ivf->shards[s], pq->shards[s], d_q, n, kk, n_probes, d_keys, st);
                    });
+}
+
+// ---- HNSW on a row-sharded set (DESIGN.md section 6): one full replica per shard entry ---------------------------------
+// A graph walk reads whichever rows the previous hop leads to, so HNSW is replicated, not sharded: replica r holds all n
+// rows and the same graph on shard r's device. A search splits its batch into contiguous slices, one per replica, and each
+// slice runs the single-GPU search on its replica: results are bit-identical to the unsharded index.
+vdb_dataset* adopt_dataset_on(int device, const void* d_rows, uint64_t n, uint32_t dim, uint32_t pitch, int dtype, int metric,
+                              uint64_t id_base);   // capi.cu
+cudaStream_t thread_stream();                      // capi.cu: the calling thread's stream on the current device
+
+}  // namespace vdb
+
+struct HnswPqReplicas {
+    uint64_t serial = 0;         // vdb_pq::serial of the row-sharded table the codes come from
+    std::vector<vdb_pq*> pq;     // pq[r]: the table's codebooks and the codes of all n rows on replica r's device
+    ~HnswPqReplicas() {
+        int prev = 0;
+        cudaGetDevice(&prev);
+        for (vdb_pq* t : pq) {
+            cudaSetDevice(t->device);
+            vdb::pq_destroy(t);
+        }
+        cudaSetDevice(prev);
+    }
+};
+
+namespace vdb {
+
+namespace {
+struct KeepDevice {   // restores the calling thread's current device on every way out
+    int prev = 0;
+    KeepDevice() { VDB_CUDA(cudaGetDevice(&prev)); }
+    ~KeepDevice() { cudaSetDevice(prev); }
+};
+}  // namespace
+
+static void free_replicas(HnswReplicas* rep) {
+    KeepDevice kd;
+    rep->pq.reset();
+    for (size_t r = 0; r < rep->ds.size(); ++r) {
+        cudaSetDevice(rep->ds[r]->device);
+        if (r < rep->h.size()) hnsw_destroy(rep->h[r]);
+        vdb_dataset_destroy(rep->ds[r]);
+    }
+    delete rep;
+}
+
+// the replicas' rows: every shard's row block is peer-copied into one buffer of all n rows on each shard entry's device
+static HnswReplicas* replicate_rows(const vdb_dataset* md) {
+    vdb_sharded_state* S = md->sharded;
+    const uint32_t G = (uint32_t)S->shards.size();
+    const uint32_t pitch = S->shards[0].ds->pitch;   // one pitch for every shard (vdb_dataset_create / _create_sharded_dev)
+    const size_t pb = (size_t)pitch * md->elem_size();
+    KeepDevice kd;
+    auto rep = new HnswReplicas();
+    rep->parent = md;
+    std::vector<cudaStream_t> st;
+    try {
+        for (uint32_t r = 0; r < G; ++r) {
+            const int dev = S->shards[r].device;
+            VDB_CUDA(cudaSetDevice(dev));
+            void* buf = nullptr;
+            VDB_CUDA(cudaMalloc(&buf, std::max<uint64_t>(md->n, 1) * pb));
+            vdb_dataset* ds = nullptr;
+            try {
+                ds = adopt_dataset_on(dev, buf, md->n, md->dim, pitch, md->dtype, md->metric, md->id_base);
+            } catch (...) {
+                cudaFree(buf);
+                throw;
+            }
+            ds->owned = true;   // vdb_dataset_destroy frees the buffer
+            rep->ds.push_back(ds);
+            st.push_back(thread_stream());
+            for (const Shard& sh : S->shards)
+                if (sh.hi > sh.lo)
+                    VDB_CUDA(cudaMemcpyPeerAsync((uint8_t*)buf + sh.lo * pb, dev, sh.ds->d_rows, sh.device, (sh.hi - sh.lo) * pb, st[r]));
+        }
+        for (uint32_t r = 0; r < G; ++r) {
+            VDB_CUDA(cudaSetDevice(rep->ds[r]->device));
+            VDB_CUDA(cudaStreamSynchronize(st[r]));
+        }
+    } catch (...) {
+        for (size_t r = 0; r < st.size(); ++r) {
+            cudaSetDevice(rep->ds[r]->device);
+            cudaStreamSynchronize(st[r]);
+        }
+        free_replicas(rep);
+        throw;
+    }
+    return rep;
+}
+
+// replicas rep->h.size() .. G-1 from a graph in host memory (the layouts of vdb_hnsw_create_from_graph)
+static void replicate_graph(HnswReplicas* rep, uint32_t M, uint32_t ef_construction, const uint32_t* h_levels, const uint32_t* links0,
+                            const uint32_t* len0, const uint32_t* ulinks, const uint32_t* ulen, int64_t enter_point,
+                            int32_t enter_level) {
+    for (size_t r = rep->h.size(); r < rep->ds.size(); ++r) {
+        VDB_CUDA(cudaSetDevice(rep->ds[r]->device));
+        rep->h.push_back(hnsw_from_graph(rep->ds[r], M, ef_construction, h_levels, links0, len0, ulinks, ulen, enter_point,
+                                         enter_level));
+    }
+}
+
+// the caller's handle: replica 0's scalars, no arrays of its own
+static vdb_hnsw* replicated_handle(HnswReplicas* rep) {
+    const vdb_hnsw* h0 = rep->h[0];
+    auto h = new vdb_hnsw();
+    h->device = h0->device;
+    h->n = h0->n;
+    h->dim = h0->dim;
+    h->dtype = h0->dtype;
+    h->metric = h0->metric;
+    h->M = h0->M;
+    h->M0 = h0->M0;
+    h->ef_construction = h0->ef_construction;
+    h->h_level = h0->h_level;
+    h->slots = h0->slots;
+    h->enter_point = h0->enter_point;
+    h->enter_level = h0->enter_level;
+    h->rep = rep;
+    return h;
+}
+
+// build once on replica 0, then every other replica loads that graph
+vdb_hnsw* sharded_hnsw_build(const vdb_dataset* md, uint32_t M, uint32_t ef_construction, const uint32_t* h_levels,
+                             uint32_t max_batch) {
+    KeepDevice kd;
+    HnswReplicas* rep = replicate_rows(md);
+    try {
+        VDB_CUDA(cudaSetDevice(rep->ds[0]->device));
+        rep->h.push_back(hnsw_build(rep->ds[0], M, ef_construction, h_levels, max_batch));
+        const vdb_hnsw* h0 = rep->h[0];
+        const uint64_t n = h0->n;
+        std::vector<uint32_t> links0(n * h0->M0), len0(n), ulinks(h0->slots * h0->M), ulen(h0->slots);
+        if (n) {
+            VDB_CUDA(cudaMemcpy(links0.data(), h0->d_links0, links0.size() * 4, cudaMemcpyDeviceToHost));
+            VDB_CUDA(cudaMemcpy(len0.data(), h0->d_len0, len0.size() * 4, cudaMemcpyDeviceToHost));
+        }
+        if (h0->slots) {
+            VDB_CUDA(cudaMemcpy(ulinks.data(), h0->d_ulinks, ulinks.size() * 4, cudaMemcpyDeviceToHost));
+            VDB_CUDA(cudaMemcpy(ulen.data(), h0->d_ulen, ulen.size() * 4, cudaMemcpyDeviceToHost));
+        }
+        replicate_graph(rep, h0->M, h0->ef_construction, h0->h_level.data(), links0.data(), len0.data(), ulinks.data(), ulen.data(),
+                        h0->enter_point, h0->enter_level);
+    } catch (...) {
+        free_replicas(rep);
+        throw;
+    }
+    return replicated_handle(rep);
+}
+
+vdb_hnsw* sharded_hnsw_from_graph(const vdb_dataset* md, uint32_t M, uint32_t ef_construction, const uint32_t* h_levels,
+                                  const uint32_t* links0, const uint32_t* len0, const uint32_t* ulinks, const uint32_t* ulen,
+                                  int64_t enter_point, int32_t enter_level) {
+    KeepDevice kd;
+    HnswReplicas* rep = replicate_rows(md);
+    try {
+        replicate_graph(rep, M, ef_construction, h_levels, links0, len0, ulinks, ulen, enter_point, enter_level);
+    } catch (...) {
+        free_replicas(rep);
+        throw;
+    }
+    return replicated_handle(rep);
+}
+
+void sharded_hnsw_destroy(vdb_hnsw* h) {
+    free_replicas(h->rep);
+    delete h;
+}
+
+// one unsharded table per replica from a row-sharded table: the same codebooks, the shards' codes in row order
+static std::shared_ptr<const HnswPqReplicas> pq_replicas(HnswReplicas* rep, const vdb_pq* pq) {
+    std::lock_guard<std::mutex> lk(rep->pq_mu);
+    if (rep->pq && rep->pq->serial == pq->serial) return rep->pq;
+    const vdb_pq* t0 = pq->shards[0];
+    std::vector<uint8_t> books((size_t)t0->kc * t0->dim * (t0->dtype == VDB_F32 ? 4 : 1));   // groups partition the dims
+    std::vector<uint8_t> codes(std::max<uint64_t>(pq->n * pq->enc, 1));
+    VDB_CUDA(cudaSetDevice(t0->device));
+    VDB_CUDA(cudaMemcpy(books.data(), t0->d_codebooks, books.size(), cudaMemcpyDeviceToHost));
+    uint64_t at = 0;
+    for (const vdb_pq* t : pq->shards) {
+        VDB_CUDA(cudaSetDevice(t->device));
+        if (t->n) VDB_CUDA(cudaMemcpy(codes.data() + at * pq->enc, t->d_codes, t->n * t->enc, cudaMemcpyDeviceToHost));
+        at += t->n;
+    }
+    auto c = std::make_shared<HnswPqReplicas>();
+    c->serial = pq->serial;
+    for (vdb_dataset* ds : rep->ds) {
+        VDB_CUDA(cudaSetDevice(ds->device));
+        c->pq.push_back(pq_create(ds, books.data(), pq->m, pq->n_bits, codes.data(), nullptr));
+    }
+    rep->pq = c;
+    return c;
+}
+
+// knn_with_ef (pq == nullptr) / knn_pq on the sharded set: min(G, nq) contiguous slices of the batch, slice i on replica
+// (first + i) % G. Every slice's upload, search and download is enqueued on the calling thread's stream of its replica's
+// device before any is waited for, so the replicas run at the same time; the call stays re-entrant (no shared state
+// but the replicas' overflow / evaluation counters, which are atomics).
+void sharded_hnsw_knn(const vdb_dataset* md, const vdb_hnsw* h, const vdb_pq* pq, const void* queries, uint32_t nq, uint32_t k,
+                      uint32_t ef, uint64_t* ids, float* dist, uint32_t* counts) {
+    HnswReplicas* rep = h->rep;
+    VDB_REQUIRE(rep && rep->parent == md && h->n == md->n, "HNSW index was built for a different vector set");
+    if (pq) {
+        VDB_REQUIRE(!pq->shards.empty() && pq->parent == md && pq->n == md->n,
+                    "PQ table was built for a different vector set (it must be rebuilt after add/delete)");
+        VDB_REQUIRE(pq->metric == md->metric, "Distance algorithm mismatch.");
+        VDB_REQUIRE(pq->n_bits == 4, "HNSW + PQ search supports 4-bit codes");
+    }
+    if (nq == 0) return;
+    if (k == 0) {
+        memset(counts, 0, (size_t)nq * 4);
+        return;
+    }
+    KeepDevice kd;
+    const std::shared_ptr<const HnswPqReplicas> pqr = pq ? pq_replicas(rep, pq) : nullptr;
+    const uint32_t G = (uint32_t)rep->h.size(), R = std::min(G, nq);
+    // calls with fewer queries than replicas start at a rotating replica, so concurrent single-query callers spread out
+    const uint32_t first = nq < G ? rep->next.fetch_add(1, std::memory_order_relaxed) % G : 0;
+    const size_t rb = (size_t)md->dim * md->elem_size();
+    struct Slice {
+        uint32_t r = 0, lo = 0, cnt = 0;
+        cudaStream_t st = nullptr;
+        DevBuf q, keys, ids, dist, counts;
+    };
+    std::vector<Slice> sl(R);
+    auto settle = [&](Slice& x) {   // waits for the slice and frees its buffers on its device
+        VDB_CUDA(cudaSetDevice(rep->ds[x.r]->device));
+        VDB_CUDA(cudaStreamSynchronize(x.st));
+        x.q = DevBuf();
+        x.keys = DevBuf();
+        x.ids = DevBuf();
+        x.dist = DevBuf();
+        x.counts = DevBuf();
+    };
+    try {
+        for (uint32_t i = 0; i < R; ++i) {
+            Slice& x = sl[i];
+            uint64_t lo, hi;
+            shard_bounds(nq, R, i, &lo, &hi);
+            x.r = (first + i) % G;
+            x.lo = (uint32_t)lo;
+            x.cnt = (uint32_t)(hi - lo);
+            const vdb_dataset* ds = rep->ds[x.r];
+            VDB_CUDA(cudaSetDevice(ds->device));
+            x.st = thread_stream();
+            x.q = DevBuf((size_t)x.cnt * rb, x.st);
+            x.keys = DevBuf((size_t)x.cnt * k * 8, x.st);
+            x.ids = DevBuf((size_t)x.cnt * k * 8, x.st);
+            x.dist = DevBuf((size_t)x.cnt * k * 4, x.st);
+            x.counts = DevBuf((size_t)x.cnt * 4, x.st);
+            VDB_CUDA(cudaMemcpyAsync(x.q.p, (const uint8_t*)queries + (size_t)x.lo * rb, (size_t)x.cnt * rb, cudaMemcpyHostToDevice,
+                                     x.st));
+            if (pq) hnsw_knn_pq_keys(ds, rep->h[x.r], pqr->pq[x.r], x.q.p, x.cnt, k, ef, x.keys.as<uint64_t>(), x.st);
+            else hnsw_knn_keys(ds, rep->h[x.r], x.q.p, x.cnt, k, ef, x.keys.as<uint64_t>(), x.st);
+            decode_keys(x.keys.as<uint64_t>(), x.cnt, k, x.ids.as<uint64_t>(), x.dist.as<float>(), x.counts.as<uint32_t>(), x.st);
+        }
+        for (Slice& x : sl) {
+            VDB_CUDA(cudaSetDevice(rep->ds[x.r]->device));
+            VDB_CUDA(cudaMemcpyAsync(ids + (size_t)x.lo * k, x.ids.p, (size_t)x.cnt * k * 8, cudaMemcpyDeviceToHost, x.st));
+            VDB_CUDA(cudaMemcpyAsync(dist + (size_t)x.lo * k, x.dist.p, (size_t)x.cnt * k * 4, cudaMemcpyDeviceToHost, x.st));
+            VDB_CUDA(cudaMemcpyAsync(counts + x.lo, x.counts.p, (size_t)x.cnt * 4, cudaMemcpyDeviceToHost, x.st));
+        }
+    } catch (...) {
+        for (Slice& x : sl)   // nothing enqueued by the call may outlive it
+            if (x.st) {
+                cudaSetDevice(rep->ds[x.r]->device);
+                cudaStreamSynchronize(x.st);
+            }
+        throw;
+    }
+    // every replica that took part has its counter read (and cleared); a full visited set on any of them fails the call
+    int code = 0;
+    std::string err;
+    for (Slice& x : sl) {
+        settle(x);
+        try {
+            hnsw_check_overflow(rep->h[x.r], x.st);
+        } catch (const Error& e) {
+            if (!code) code = e.code, err = e.what();
+        }
+    }
+    if (code) throw Error(code, err);
 }
 
 uint32_t sharded_count(const vdb_dataset* md) { return md->sharded ? (uint32_t)md->sharded->shards.size() : 0; }

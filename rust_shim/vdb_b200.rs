@@ -11,7 +11,8 @@
 //!   KMeans::from_vec_set / find_nearest   -> gpu_kmeans_from_vec_set / gpu_find_nearest_batch (src/distance/k_means.rs)
 //!   PQTable::from_vec_set                 -> gpu_pq_table_from_vec_set            (src/distance/pq_table.rs:141-191)
 //! behind the same traits (src/index_algorithm/mod.rs:35-154). With `gpu_init(&[0,1,..,7])` called once, the same
-//! `knn` call runs row-sharded on every listed GPU (one C call, per-GPU top-k merged over NVLink peer memory).
+//! `knn` call runs row-sharded on every listed GPU (one C call, per-GPU top-k merged over NVLink peer memory); HNSW
+//! keeps a replica per GPU and splits the query batch over them.
 #![allow(non_camel_case_types)]
 use std::os::raw::{c_char, c_int, c_void};
 use std::sync::Mutex;
@@ -347,7 +348,8 @@ impl<T: Scalar> IndexPQ<T> for GpuIvfIndex<T> {
 // ------------------------------------------------------------------------------------------------ HNSW
 /// Drop-in for `HNSWIndex<T>` (hnsw_index.rs:99-141). The graph lives on the device in the reference's own layout;
 /// `to_host` copies it into an `HNSWIndex<T>` (bincode save, IndexSerdeExternalVecSet :641-668) and `from_host`
-/// mirrors a loaded one.
+/// mirrors a loaded one. After `gpu_init` with several GPUs every GPU holds a replica of the rows and the graph, and each
+/// `knn` / `knn_pq` batch is split over them in one call, with the single-GPU results; `batch_add` is refused there.
 pub struct GpuHnswIndex<T: Scalar> {
     pub dist: DistanceAlgorithm,
     pub vec_set: VecSet<T>,
