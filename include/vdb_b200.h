@@ -101,7 +101,10 @@ int vdb_gather_dist(const vdb_dataset* ds, const void* queries, uint32_t nq, con
 /* IndexKNN::knn for FlatIndex (src/index_algorithm/flat_index.rs:48-57), batched over nq queries
  * (nq == 1 is the unchanged trait call; nq > 1 is the additive batch entry used by bench drivers,
  * examples/bench.rs:414-418, src/bin/gen_gnd.rs:65-68). Exact: the k smallest by (distance, id),
- * distances in the difference form sum((q-x)^2) / the 3-dot cosine form. */
+ * distances in the difference form sum((q-x)^2) / the 3-dot cosine form. Any k: counts = min(k, n), slots past it hold
+ * id UINT64_MAX and a NaN distance. Above the fused shared-memory top-k (about 15 900) the call keys every row and selects +
+ * sorts in global memory, chunked so device scratch stays bounded (INTEGRATION.md section 4); its first columns are the
+ * bits of the call at a smaller k. */
 int vdb_flat_knn(const vdb_dataset* ds, const void* queries, uint32_t nq, uint32_t k, uint64_t* ids,
                  float* dist, uint32_t* counts);
 int vdb_flat_knn_dev(const vdb_dataset* ds, const void* d_queries, uint32_t nq, uint32_t k,
@@ -109,7 +112,7 @@ int vdb_flat_knn_dev(const vdb_dataset* ds, const void* d_queries, uint32_t nq, 
 /* The same on a row-sharded set with the batch already resident on every shard's device: d_queries[s] = the whole
  * [nq, dim] batch on shard s's device. Shard s OWNS the queries [s * per, min(nq, (s + 1) * per)), per = ceil(nq / G),
  * and receives their merged results in d_ids[s] / d_dist[s] / d_counts[s] (arrays of at least `per` rows on its
- * device). nq <= 16384 per call. Synchronous: every shard's stream has drained on return. */
+ * device). nq <= 16384 per call, any k. Synchronous: every shard's stream has drained on return. */
 int vdb_flat_knn_sharded_dev(const vdb_dataset* ds, const void* const* d_queries, uint32_t nq, uint32_t k,
                              uint64_t* const* d_ids, float* const* d_dist, uint32_t* const* d_counts);
 /* Concurrent nq == 1 calls of vdb_flat_knn on one handle - the reference's call pattern: one query per knn call from

@@ -467,6 +467,8 @@ int vdb_dataset_destroy(vdb_dataset* ds) {
 }
 
 // ---- Flat ------------------------------------------------------------------------------------------
+constexpr uint64_t LARGE_K_RESULT_BYTES = 1ull << 30;
+
 int vdb_flat_set_path(int path) {
     return guarded([&] {
         VDB_REQUIRE(path >= 0 && path <= 2, "path must be 0 (auto), 1 (scan) or 2 (tensor)");
@@ -654,17 +656,30 @@ int vdb_flat_knn(const vdb_dataset* ds, const void* queries, uint32_t nq, uint32
             vdb::sharded_flat_knn(ds, queries, nq, k, ids, dist, counts);
             return;
         }
-        if (nq == 1 && k > 0 && ds->n > 0 && vdb::g_batching.load()) {   // the trait's call: coalesced with concurrent callers
+        // the trait's call: coalesced with concurrent callers, unless k is above the fused top-k (the batcher's page-locked
+        // staging would grow with k, and such a call is a pass of its own)
+        if (nq == 1 && k > 0 && ds->n > 0 && vdb::g_batching.load() && vdb::fused_topk_fits(ds, 1, k)) {
             batched_single_knn(ds, queries, k, ids, dist, counts);
             return;
         }
-        host_search(dev_of(ds), queries, nq, (size_t)ds->dim * ds->elem_size(), k, ids, dist, counts,
-                    [&](void* dq, uint64_t* dids, float* dd, uint32_t* dc, cudaStream_t st) {
-                        vdb::DevBuf keys((size_t)nq * k * 8, st);
-                        const vdb::ScanOut so{dids, dd, dc};
-                        if (!flat_keys_dispatch(ds, dq, nq, k, keys.as<uint64_t>(), st, &so))
-                            vdb::decode_keys(keys.as<uint64_t>(), nq, k, dids, dd, dc, st);
-                    });
+        const size_t qb = (size_t)ds->dim * ds->elem_size();
+        auto search = [&](uint32_t q0, uint32_t n) {
+            host_search(dev_of(ds), (const uint8_t*)queries + (size_t)q0 * qb, n, qb, k, ids + (size_t)q0 * k,
+                        dist + (size_t)q0 * k, counts + q0, [&](void* dq, uint64_t* dids, float* dd, uint32_t* dc, cudaStream_t st) {
+                            vdb::DevBuf keys((size_t)n * k * 8, st);
+                            const vdb::ScanOut so{dids, dd, dc};
+                            if (!flat_keys_dispatch(ds, dq, n, k, keys.as<uint64_t>(), st, &so))
+                                vdb::decode_keys(keys.as<uint64_t>(), n, k, dids, dd, dc, st);
+                        });
+        };
+        if (vdb::fused_topk_fits(ds, nq, k)) {
+            search(0, nq);
+            return;
+        }
+        // large k: the device copies of the results (keys, ids, distances: 20 bytes per slot) take at most
+        // LARGE_K_RESULT_BYTES per pass, at least one query
+        const uint32_t chunk = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(nq, LARGE_K_RESULT_BYTES / ((uint64_t)k * 20)));
+        for (uint32_t q0 = 0; q0 < nq; q0 += chunk) search(q0, std::min(chunk, nq - q0));
     });
 }
 

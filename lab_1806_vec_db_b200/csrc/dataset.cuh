@@ -66,6 +66,9 @@ struct ScanOut {
     float* dist = nullptr;
     uint32_t* counts = nullptr;
 };
+// True when the fused top-k of the scan holds k (its shared-memory segments and, when the per-CTA lists are merged, the
+// merge's); otherwise flat_scan_keys takes the large-k path (emit every key, then select + sort in global memory).
+bool fused_topk_fits(const vdb_dataset* ds, uint32_t nq, uint32_t k);
 bool flat_scan_keys(const vdb_dataset* ds, const void* d_queries, uint32_t nq, uint32_t k, uint64_t* d_keys, cudaStream_t st,
                     const ScanOut* out = nullptr);
 // decode [nq][k] keys into the SoA result arrays

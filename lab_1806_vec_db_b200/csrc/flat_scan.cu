@@ -45,6 +45,7 @@ struct ScanParams {
     uint64_t* out_ids;     // optional decoded results
     float* out_dist;
     uint32_t* out_counts;
+    uint64_t* emit;        // emit instantiation only: [nq_valid][n] the key of every (query, row), see flat_large_k_keys
 };
 
 // Tail of a single-launch batch, run by the last CTA to finish: merge of the gridDim.x per-CTA lists of every query + decode.
@@ -114,8 +115,10 @@ static __device__ __noinline__ void scan_tail(const ScanTailArgs p, TopkSmem top
     if (p.out_counts && threadIdx.x < p.nq_valid) p.out_counts[threadIdx.x] = s_valid[threadIdx.x];
 }
 
-// PL = 1: f32 rows (4 elements per 16-byte load); PL = 4: u8 rows (16 elements per load)
-template <int NQ, int R, int METRIC, int PL>
+// PL = 1: f32 rows (4 elements per 16-byte load); PL = 4: u8 rows (16 elements per load).
+// EMIT: the large-k path's instantiation - every key goes to p.emit instead of the shared-memory top-k (a compile-time
+// switch: the distance code is the same, and the top-k instantiations keep their register allocation).
+template <int NQ, int R, int METRIC, int PL, bool EMIT = false>
 __global__ void __launch_bounds__(SCAN_THREADS, 2) flat_scan_kernel(const ScanParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     constexpr int V = NQ * R;
@@ -141,7 +144,8 @@ __global__ void __launch_bounds__(SCAN_THREADS, 2) flat_scan_kernel(const ScanPa
         for (uint32_t i = threadIdx.x; i < NQ * qs4; i += blockDim.x)
             qs[i] = (i / qs4 < p.nq_valid) ? reinterpret_cast<const float4*>(p.q)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    topk.init();
+    if constexpr (EMIT) __syncthreads();
+    else topk.init();
 
     const int pidx = lane >> SH;
     const int my_r = pidx / NQ, my_q = pidx % NQ;
@@ -293,9 +297,10 @@ __global__ void __launch_bounds__(SCAN_THREADS, 2) flat_scan_kernel(const ScanPa
         const uint64_t row = g * R + my_r;
         if (emitter && row < p.n) {
             const uint64_t key = make_key(tot, p.id_base + (uint32_t)row);
-            if (key < topk.tau(my_q)) want |= topk.push(my_q, key);
+            if constexpr (EMIT) p.emit[(size_t)my_q * p.n + row] = key;
+            else if (key < topk.tau(my_q)) want |= topk.push(my_q, key);
         }
-        if ((gi + 1) % p.sync_every == 0) {
+        if (!EMIT && (gi + 1) % p.sync_every == 0) {
             topk.maybe_flush(want);
             want = false;
         }
@@ -344,6 +349,7 @@ __global__ void __launch_bounds__(SCAN_THREADS, 2) flat_scan_kernel(const ScanPa
             }
         }
     }
+    if constexpr (EMIT) return;
     topk.final_flush();
     for (uint32_t i = threadIdx.x; i < p.nq_valid * p.K; i += blockDim.x) {
         const uint32_t qi = i / p.K, j = i - qi * p.K;
@@ -458,6 +464,10 @@ __global__ void __launch_bounds__(MERGE_THREADS, 8) merge_keys_kernel(
     }
 }
 
+constexpr size_t MERGE_SMEM_MAX = 200 * 1024;
+// the check of launch_merge_keys below for an input of more than 1024 keys per query (shorter inputs always fit)
+bool merge_keys_fits(uint32_t k) { return TopkSmem::bytes(1, topk_segment_size(k, MERGE_THREADS)) <= MERGE_SMEM_MAX; }
+
 void launch_merge_keys(const uint64_t* d_keys, uint32_t nlists, uint32_t nq, uint32_t len, bool list_major,
                        uint32_t k, uint64_t* d_out_keys, uint64_t* d_ids, float* d_dist,
                        uint32_t* d_counts, cudaStream_t stream, const uint64_t* d_seg_off, const uint32_t* d_seg_cnt,
@@ -475,7 +485,7 @@ void launch_merge_keys(const uint64_t* d_keys, uint32_t nlists, uint32_t nq, uin
         limit = P - k - MERGE_THREADS;
     }
     const size_t smem = TopkSmem::bytes(1, P);
-    VDB_REQUIRE(smem <= 200 * 1024, "k=%u too large for the fused top-k (max %u)", k, 20000u);
+    VDB_REQUIRE(smem <= MERGE_SMEM_MAX, "k=%u too large for the fused top-k (max %u)", k, 20000u);
     if (smem > 48 * 1024)
         VDB_CUDA(cudaFuncSetAttribute(merge_keys_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)smem));
@@ -556,10 +566,14 @@ __global__ void __launch_bounds__(256) merge_sorted_kernel(const uint64_t* __res
 }
 
 // list-major [nlists][nq][len] ascending lists -> the k smallest per query; falls back to the generic merge when the
-// lists of a query do not fit in shared memory
+// lists of a query do not fit in shared memory, and to select + sort in global memory when k does not fit the generic merge
 void launch_merge_sorted(const uint64_t* d_keys, uint32_t nlists, uint32_t nq, uint32_t len, uint32_t k, uint64_t* d_out_keys,
                          uint64_t* d_ids, float* d_dist, uint32_t* d_counts, cudaStream_t stream) {
     if (nq == 0 || k == 0) return;
+    if (!merge_keys_fits(k)) {
+        large_k_select(d_keys, nlists, nq, len, k, d_out_keys, d_ids, d_dist, d_counts, stream);
+        return;
+    }
     static const int generic = getenv("VDB_MERGE_GENERIC") ? atoi(getenv("VDB_MERGE_GENERIC")) : 0;
     const size_t smem = ((size_t)nlists * len + k) * 8;
     if (generic || nlists == 1 || smem > 96 * 1024) {
@@ -688,28 +702,124 @@ QueryTile prepare_queries(const vdb_dataset* ds, const void* d_queries, uint32_t
 }
 
 // ---- host launcher ------------------------------------------------------------------------------
-template <int NQ, int R, int METRIC, int PL>
+template <int NQ, int R, int METRIC, int PL, bool EMIT>
 static void launch_scan(const ScanParams& p, uint32_t grid, size_t smem, cudaStream_t st) {
-    auto kern = flat_scan_kernel<NQ, R, METRIC, PL>;
+    auto kern = flat_scan_kernel<NQ, R, METRIC, PL, EMIT>;
     static std::atomic<size_t> configured[VDB_MAX_DEVICES];
     if (smem > 48 * 1024) ensure_dyn_smem(kern, smem, configured);
-    ProfScope prof("flat_scan", st);
+    ProfScope prof(EMIT ? "flat_scan_emit" : "flat_scan", st);
     kern<<<grid, SCAN_THREADS, smem, st>>>(p);
     VDB_LAUNCHED();
 }
 
-template <int METRIC, int PL>
+template <int METRIC, int PL, bool EMIT = false>
 static void dispatch_scan(int nqt, const ScanParams& p, uint32_t grid, size_t smem, cudaStream_t st) {
     switch (nqt) {
-        case 1: launch_scan<1, 8, METRIC, PL>(p, grid, smem, st); break;
-        case 2: launch_scan<2, 8, METRIC, PL>(p, grid, smem, st); break;
-        case 4: launch_scan<4, 4, METRIC, PL>(p, grid, smem, st); break;
-        default: launch_scan<8, 4, METRIC, PL>(p, grid, smem, st); break;
+        case 1: launch_scan<1, 8, METRIC, PL, EMIT>(p, grid, smem, st); break;
+        case 2: launch_scan<2, 8, METRIC, PL, EMIT>(p, grid, smem, st); break;
+        case 4: launch_scan<4, 4, METRIC, PL, EMIT>(p, grid, smem, st); break;
+        default: launch_scan<8, 4, METRIC, PL, EMIT>(p, grid, smem, st); break;
+    }
+}
+template <bool EMIT = false>
+static void dispatch_scan_ds(const vdb_dataset* ds, int nqt, const ScanParams& p, uint32_t grid, size_t smem, cudaStream_t st) {
+    if (ds->dtype == VDB_F32) {
+        if (ds->metric == VDB_L2SQR) dispatch_scan<VDB_L2SQR, 1, EMIT>(nqt, p, grid, smem, st);
+        else dispatch_scan<VDB_COSINE, 1, EMIT>(nqt, p, grid, smem, st);
+    } else {
+        if (ds->metric == VDB_L2SQR) dispatch_scan<VDB_L2SQR, 4, EMIT>(nqt, p, grid, smem, st);
+        else dispatch_scan<VDB_COSINE, 4, EMIT>(nqt, p, grid, smem, st);
     }
 }
 static int rows_per_group(int nqt) { return nqt <= 2 ? 8 : 4; }
+// query tile + top-k segments (P = 0: the emit instantiation, no segments)
+static size_t scan_smem(const QueryTile& qt, int nqt, uint32_t P) {
+    return (size_t)nqt * qt.qstride * 4 + (P ? TopkSmem::bytes(nqt, P) : 0);
+}
 
 constexpr size_t SCAN_SMEM_MAX = 200 * 1024;
+
+// The CTA-wide flush test (a barrier) runs every `sync_every` row groups: often enough that a query's segment cannot
+// overflow between two tests (at most `period` appends), but not more often than every ~8 steps of 512 bytes - short
+// rows (u8 x 960 = 2 steps per group, 128-d f32 = 1) otherwise meet at a barrier after every group and lose the overlap
+// between warps (measured neutral for u8 x 960, where something else bounds the pass at 0.253 ms).
+static uint32_t sync_every_for(uint32_t nit, uint32_t R) {
+    return std::max(std::max(1u, 64u / (SCAN_WARPS * R)), ceil_div(8u, nit));
+}
+// shared memory of the fused scan: the top-k segment size and the largest query template (<= 8) that fits
+struct ScanFit {
+    uint32_t period, P;
+    int nqt;
+    bool fits;
+};
+static ScanFit scan_fit(const QueryTile& qt, uint32_t k) {
+    ScanFit f;
+    f.period = std::max(sync_every_for(qt.nit, 4) * SCAN_WARPS * 4, sync_every_for(qt.nit, 8) * SCAN_WARPS * 8);
+    f.P = topk_segment_size(k, f.period);
+    f.nqt = 8;
+    while (f.nqt > 1 && scan_smem(qt, f.nqt, f.P) > SCAN_SMEM_MAX) f.nqt >>= 1;
+    f.fits = scan_smem(qt, f.nqt, f.P) <= SCAN_SMEM_MAX;
+    return f;
+}
+static bool scan_fuse_on() {
+    const char* fuse_s = getenv("VDB_SCAN_FUSE");   // read per call: the tests toggle it in one process
+    return !(fuse_s && !atoi(fuse_s));
+}
+
+bool fused_topk_fits(const vdb_dataset* ds, uint32_t nq, uint32_t k) {
+    if (nq == 0 || k == 0 || ds->n == 0) return true;
+    const ScanFit f = scan_fit(query_tile_shape(ds), k);
+    if (!f.fits) return false;
+    // the per-CTA lists are merged by launch_merge_keys unless the whole batch is one launch with the fused tail
+    const bool merged = !(scan_fuse_on() && nq <= 8 && nq <= (uint32_t)f.nqt);
+    return !merged || merge_keys_fits(k);
+}
+
+// Large-k path: the emit instantiation of the scan writes the key of every (query, row) of a chunk of queries to global
+// memory - one rows pass per <= 8 queries, as in the fused scan - and large_k_select reduces each query's n keys to its
+// k best. Emitted keys take at most LARGE_K_EMIT_BYTES per chunk (at least one query).
+constexpr uint64_t LARGE_K_EMIT_BYTES = 1ull << 30;
+static void flat_large_k_keys(const vdb_dataset* ds, const void* d_queries, uint32_t nq, uint32_t k, uint64_t* d_keys,
+                              cudaStream_t st) {
+    const QueryTile qt = prepare_queries(ds, d_queries, nq, st);
+    int nqt = 8;
+    while (nqt > 1 && scan_smem(qt, nqt, 0) > SCAN_SMEM_MAX) nqt >>= 1;
+    VDB_REQUIRE(scan_smem(qt, nqt, 0) <= SCAN_SMEM_MAX, "flat scan: dim=%u does not fit in shared memory", ds->dim);
+    const uint64_t per_query = ds->n * 8;
+    uint32_t chunk = (uint32_t)std::min<uint64_t>(nq, std::max<uint64_t>(1, LARGE_K_EMIT_BYTES / per_query));
+    if (chunk > 8) chunk = chunk / 8 * 8;   // whole 8-query passes
+    DevBuf emit((size_t)chunk * per_query, st);
+    const int sms = sm_count();
+    ScanParams p{};
+    p.rows = (const uint8_t*)ds->d_rows;
+    p.n = ds->n;
+    p.pitch_bytes = ds->pitch_bytes();
+    p.nvec = qt.nvec;
+    p.nit = qt.nit;
+    p.qstride = qt.qstride;
+    p.raw_dim = ds->dim;
+    p.sync_every = 1;
+    p.id_base = (uint32_t)ds->id_base;
+    for (uint32_t q0 = 0; q0 < nq; q0 += chunk) {
+        const uint32_t qn = std::min(chunk, nq - q0);
+        for (uint32_t qq = 0; qq < qn;) {
+            const uint32_t left = qn - qq;
+            int t = nqt;
+            while (t > 1 && (uint32_t)(t >> 1) >= left) t >>= 1;
+            const uint32_t now = std::min<uint32_t>(left, t);
+            const uint64_t ngroups = ceil_div<uint64_t>(ds->n, rows_per_group(t));
+            const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(2 * sms, ceil_div<uint64_t>(ngroups, SCAN_WARPS)));
+            p.iters = (uint32_t)ceil_div<uint64_t>(ngroups, (uint64_t)grid * SCAN_WARPS);
+            p.q = qt.q.as<float>() + (size_t)(q0 + qq) * qt.qstride;
+            p.qcache = qt.qcache.as<float>() + (q0 + qq);
+            p.nq_valid = now;
+            p.emit = emit.as<uint64_t>() + (size_t)qq * ds->n;
+            dispatch_scan_ds<true>(ds, t, p, grid, scan_smem(qt, t, 0), st);
+            qq += now;
+        }
+        large_k_select(emit.as<uint64_t>(), 1, qn, ds->n, k, d_keys + (size_t)q0 * k, nullptr, nullptr, nullptr, st);
+    }
+}
 
 bool flat_scan_keys(const vdb_dataset* ds, const void* d_queries, uint32_t nq, uint32_t k,
                     uint64_t* d_keys, cudaStream_t st, const ScanOut* out) {
@@ -718,8 +828,11 @@ bool flat_scan_keys(const vdb_dataset* ds, const void* d_queries, uint32_t nq, u
         VDB_CUDA(cudaMemsetAsync(d_keys, 0xff, (size_t)nq * k * 8, st));
         return false;
     }
-    const char* fuse_s = getenv("VDB_SCAN_FUSE");   // read per call: the tests toggle it in one process
-    const bool fuse_on = !(fuse_s && !atoi(fuse_s));
+    if (!fused_topk_fits(ds, nq, k)) {
+        flat_large_k_keys(ds, d_queries, nq, k, d_keys, st);
+        return false;
+    }
+    const bool fuse_on = scan_fuse_on();
     DevBuf done(fuse_on && nq <= 8 ? 4 : 0, st);   // arrival counter of the fused tail (cleared by the tile kernel)
     // u8 rows under L2Sqr in one launch (the trait's single-query call): the scan CTAs read the caller's query bytes
     // themselves and the counter is cleared by a 4-byte memset - no tile kernel in front of the scan
@@ -733,21 +846,11 @@ bool flat_scan_keys(const vdb_dataset* ds, const void* d_queries, uint32_t nq, u
         qt = prepare_queries(ds, d_queries, nq, st, done.as<uint32_t>());
     }
 
-    // queries per pass: as many as fit (<= 8) next to the top-k segments in shared memory.
-    // The CTA-wide flush test (a barrier) runs every `sync_every` row groups: often enough that a query's segment
-    // cannot overflow between two tests (at most `period` appends), but not more often than every ~8 steps of 512
-    // bytes - short rows (u8 x 960 = 2 steps per group, 128-d f32 = 1) otherwise meet at a barrier after every group
-    // and lose the overlap between warps (measured neutral for u8 x 960, where something else bounds the pass at 0.253 ms).
-    auto sync_for = [&](uint32_t R) {
-        return std::max(std::max(1u, 64u / (SCAN_WARPS * R)), ceil_div(8u, qt.nit));
-    };
-    const uint32_t period = std::max(sync_for(4) * SCAN_WARPS * 4, sync_for(8) * SCAN_WARPS * 8);
-    const uint32_t P = topk_segment_size(k, period);
-    int nqt = 8;
-    auto smem_for = [&](int t) { return (size_t)t * qt.qstride * 4 + TopkSmem::bytes(t, P); };
-    while (nqt > 1 && smem_for(nqt) > SCAN_SMEM_MAX) nqt >>= 1;
-    VDB_REQUIRE(smem_for(nqt) <= SCAN_SMEM_MAX,
-                "flat scan: dim=%u with k=%u does not fit in shared memory", ds->dim, k);
+    // queries per pass: as many as fit (<= 8) next to the top-k segments in shared memory (fused_topk_fits held)
+    const ScanFit fit = scan_fit(qt, k);
+    const uint32_t period = fit.period, P = fit.P;
+    const int nqt = fit.nqt;
+    auto smem_for = [&](int t) { return scan_smem(qt, t, P); };
 
     const int sms = sm_count();
     ScanParams p{};
@@ -785,7 +888,7 @@ bool flat_scan_keys(const vdb_dataset* ds, const void* d_queries, uint32_t nq, u
             // every pass of a chunk must use the same grid so the partial layout is uniform
             if (grid_used == 0) grid_used = grid;
             p.iters = (uint32_t)ceil_div<uint64_t>(ngroups, (uint64_t)grid_used * SCAN_WARPS);
-            p.sync_every = sync_for((uint32_t)R);
+            p.sync_every = sync_every_for(qt.nit, (uint32_t)R);
             p.q = raw_q ? nullptr : qt.q.as<float>() + (size_t)(q0 + qq) * qt.qstride;
             p.qcache = raw_q ? nullptr : qt.qcache.as<float>() + (q0 + qq);
             p.raw_q = raw_q ? (const uint8_t*)d_queries + (size_t)(q0 + qq) * ds->dim : nullptr;
@@ -799,14 +902,7 @@ bool flat_scan_keys(const vdb_dataset* ds, const void* d_queries, uint32_t nq, u
             p.out_ids = fused && out ? out->ids : nullptr;
             p.out_dist = fused && out ? out->dist : nullptr;
             p.out_counts = fused && out ? out->counts : nullptr;
-            const size_t smem = smem_for(t);
-            if (ds->dtype == VDB_F32) {
-                if (ds->metric == VDB_L2SQR) dispatch_scan<VDB_L2SQR, 1>(t, p, grid_used, smem, st);
-                else dispatch_scan<VDB_COSINE, 1>(t, p, grid_used, smem, st);
-            } else {
-                if (ds->metric == VDB_L2SQR) dispatch_scan<VDB_L2SQR, 4>(t, p, grid_used, smem, st);
-                else dispatch_scan<VDB_COSINE, 4>(t, p, grid_used, smem, st);
-            }
+            dispatch_scan_ds(ds, t, p, grid_used, smem_for(t), st);
             qq += now;
         }
         if (!fused)

@@ -727,6 +727,13 @@ static void sharded_flat_chunk(const vdb_dataset* md, const FlatCallArgs& a, int
 
 static int effective_path(const vdb_dataset* md) { return md->flat_path >= 0 ? md->flat_path : g_flat_path.load(); }
 
+// Queries per sharded Flat chunk. Above the fused top-k (the owners' merge runs in global memory) the per-shard keys and
+// the owners' merge inputs, nq * k * 8 bytes each, stay within 1 GiB.
+static uint32_t shard_query_chunk(uint32_t k) {
+    if (merge_keys_fits(k)) return SHARD_QUERY_CHUNK;
+    return (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(SHARD_QUERY_CHUNK, (1ull << 30) / ((uint64_t)k * 8)));
+}
+
 // IndexKNN::knn on the sharded set, host buffers (the call a Rust host makes, whatever the GPU count)
 void sharded_flat_knn(const vdb_dataset* md, const void* queries, uint32_t nq, uint32_t k, uint64_t* ids, float* dist,
                       uint32_t* counts) {
@@ -739,9 +746,10 @@ void sharded_flat_knn(const vdb_dataset* md, const void* queries, uint32_t nq, u
     std::lock_guard<std::mutex> lk(S->call_mu);
     const size_t rb = (size_t)md->dim * md->elem_size();
     const int path = effective_path(md);
-    for (uint32_t q0 = 0; q0 < nq; q0 += SHARD_QUERY_CHUNK) {
+    const uint32_t chunk = shard_query_chunk(k);
+    for (uint32_t q0 = 0; q0 < nq; q0 += chunk) {
         FlatCallArgs a;
-        a.nq = std::min(SHARD_QUERY_CHUNK, nq - q0);
+        a.nq = std::min(chunk, nq - q0);
         a.k = k;
         a.h_queries = (const uint8_t*)queries + (size_t)q0 * rb;
         a.h_ids = ids + (size_t)q0 * k;
@@ -760,14 +768,62 @@ void sharded_flat_knn_dev(const vdb_dataset* md, const void* const* d_queries, u
     VDB_REQUIRE(k > 0, "k must be > 0");
     VDB_REQUIRE(nq <= SHARD_QUERY_CHUNK, "device-resident sharded search: at most %u queries per call", SHARD_QUERY_CHUNK);
     std::lock_guard<std::mutex> lk(S->call_mu);
-    FlatCallArgs a;
-    a.nq = nq;
-    a.k = k;
-    a.d_queries = d_queries;
-    a.d_ids = d_ids;
-    a.d_dist = d_dist;
-    a.d_counts = d_counts;
-    sharded_flat_chunk(md, a, effective_path(md));
+    const uint32_t chunk = shard_query_chunk(k);
+    if (nq <= chunk) {
+        FlatCallArgs a;
+        a.nq = nq;
+        a.k = k;
+        a.d_queries = d_queries;
+        a.d_ids = d_ids;
+        a.d_dist = d_dist;
+        a.d_counts = d_counts;
+        sharded_flat_chunk(md, a, effective_path(md));
+        return;
+    }
+    // large k, more queries than one chunk: every chunk's owners write to their staging buffers, whose rows are then
+    // copied to the owners of the whole call (query q -> shard q / per, row q % per)
+    const uint32_t G = (uint32_t)S->shards.size(), per = ceil_div(nq, G);
+    const size_t rb = (size_t)md->dim * md->elem_size();
+    std::vector<const void*> qs(G);
+    std::vector<uint64_t*> o_ids(G);
+    std::vector<float*> o_dist(G);
+    std::vector<uint32_t*> o_cnt(G);
+    int prev = 0;
+    VDB_CUDA(cudaGetDevice(&prev));
+    for (uint32_t q0 = 0; q0 < nq; q0 += chunk) {
+        const uint32_t cn = std::min(chunk, nq - q0), per_c = ceil_div(cn, G);
+        for (uint32_t s = 0; s < G; ++s) {
+            Shard& sh = S->shards[s];
+            VDB_CUDA(cudaSetDevice(sh.device));
+            sh.out_ids.ensure((size_t)per_c * k * 8);
+            sh.out_dist.ensure((size_t)per_c * k * 4);
+            sh.out_cnt.ensure((size_t)per_c * 4);
+            qs[s] = (const uint8_t*)d_queries[s] + (size_t)q0 * rb;
+            o_ids[s] = (uint64_t*)sh.out_ids.p;
+            o_dist[s] = (float*)sh.out_dist.p;
+            o_cnt[s] = (uint32_t*)sh.out_cnt.p;
+        }
+        VDB_CUDA(cudaSetDevice(prev));
+        FlatCallArgs a;
+        a.nq = cn;
+        a.k = k;
+        a.d_queries = qs.data();
+        a.d_ids = o_ids.data();
+        a.d_dist = o_dist.data();
+        a.d_counts = o_cnt.data();
+        sharded_flat_chunk(md, a, effective_path(md));   // ends with every shard's stream synchronised
+        for (uint32_t hc = 0; hc < G; ++hc) {
+            const uint32_t lo_c = std::min(cn, hc * per_c), hi_c = std::min(cn, (hc + 1) * per_c);
+            for (uint32_t q = q0 + lo_c; q < q0 + hi_c;) {
+                const uint32_t h = q / per, e = std::min(q0 + hi_c, (h + 1) * per), r = q - h * per, src = q - q0 - lo_c;
+                const size_t n = e - q;
+                VDB_CUDA(cudaMemcpy(d_ids[h] + (size_t)r * k, o_ids[hc] + (size_t)src * k, n * k * 8, cudaMemcpyDefault));
+                VDB_CUDA(cudaMemcpy(d_dist[h] + (size_t)r * k, o_dist[hc] + (size_t)src * k, n * k * 4, cudaMemcpyDefault));
+                VDB_CUDA(cudaMemcpy(d_counts[h] + r, o_cnt[hc] + src, n * 4, cudaMemcpyDefault));
+                q = e;
+            }
+        }
+    }
 }
 
 // ---- row-sharded IVF (SURVEY.md 8e): centroids replicated, every shard holds its slice of every list -------------------

@@ -98,6 +98,12 @@ struct MergeFinish {
     uint32_t* redo = nullptr;
     uint32_t* nredo = nullptr;           // zeroed by the caller
 };
+// true when launch_merge_keys holds k in shared memory (k <= 15 872); above, launch_merge_sorted uses large_k_select
+bool merge_keys_fits(uint32_t k);
+// topk_large.cu: the k smallest of the nlists * len keys per query of list-major lists [nlists][nq][len] (any order,
+// KEY_NONE entries ignored), ascending and KEY_NONE padded to k, by select + sort in global memory; any k
+void large_k_select(const uint64_t* d_keys, uint32_t nlists, uint32_t nq, uint64_t len, uint32_t k, uint64_t* d_out_keys,
+                    uint64_t* d_ids, float* d_dist, uint32_t* d_counts, cudaStream_t st);
 void launch_merge_keys(const uint64_t* d_keys, uint32_t nlists, uint32_t nq, uint32_t len, bool list_major,
                        uint32_t k, uint64_t* d_out_keys, uint64_t* d_ids, float* d_dist,
                        uint32_t* d_counts, cudaStream_t stream, const uint64_t* d_seg_off = nullptr,
