@@ -339,7 +339,9 @@ __global__ void __launch_bounds__(HN_THREADS, 4) hnsw_search_kernel(const HnswSe
                         bool fresh = false;
                         uint32_t id = 0;
                         if (j < len) {
-                            if (s_hcount + base < hlimit) {
+                            // at most one insertion per lane of this round: the set never holds more than hlimit ids,
+                            // so hash_insert always finds a free slot, whatever the set's size
+                            if (s_hcount + base + (uint32_t)lane < hlimit) {
                                 id = lk[j];
                                 fresh = hash_insert(hash, p.hash_mask, id);
                             } else {
@@ -602,9 +604,12 @@ __global__ void iota_pairs_kernel(const uint64_t* __restrict__ keys, uint32_t nq
 // ---- host side -----------------------------------------------------------------------------------------------------
 // Visited-set capacity. The reference's visited set is unbounded (hnsw_index.rs:258-291); here a search records at
 // most 2M nodes per expansion and typically 10-15. Up to ef = 896 the set lives in shared memory (8192 / 16384 / 32768
-// slots); beyond it lives in global memory with 4 ef 2M slots per CTA - room for 3.5 ef expansions of 2M fresh
-// neighbours each before the 7/8 fill limit, which a search that expands about ef entries cannot approach. A neighbour
-// that still cannot be recorded is counted (HnswSearchParams::overflow) and the call fails instead of losing recall.
+// slots); beyond it lives in global memory with 4 ef 2M slots per CTA. A neighbour that cannot be recorded because the
+// set is 7/8 full is counted (HnswSearchParams::overflow). Long walks on large hard sets do fill the smaller tiers
+// (50 000 uniform 64-d rows at M = 32 evaluate more than 7168 distinct rows at ef 200), so the host calls and every
+// build batch re-run a search that overflowed with a set that cannot fill (never_full_slots); the set's size never
+// changes a result, only whether the walk could finish. The `_dev` searches leave the count to the caller
+// (vdb_hnsw_overflow).
 constexpr uint32_t HN_SMEM_HASH_MAX_EF = 896;
 static uint32_t hash_cap_for(uint32_t ef, uint32_t M0) {
     static const uint32_t small_to = getenv("VDB_HNSW_SMALL_HASH_EF") ? (uint32_t)atoi(getenv("VDB_HNSW_SMALL_HASH_EF")) : 448u;
@@ -614,6 +619,13 @@ static uint32_t hash_cap_for(uint32_t ef, uint32_t M0) {
     if (ef <= 640) return 16384u;
     if (ef <= HN_SMEM_HASH_MAX_EF) return 32768u;
     return next_pow2(4u * ef * std::max(M0, 1u));
+}
+// slots of a visited set that one walk over n rows can never fill to 7/8: at least 8/7 (n + 1)
+static uint32_t never_full_slots(uint64_t n) {
+    const uint64_t need = (8 * (n + 1) + 6) / 7;
+    uint64_t s = 1;
+    while (s < need) s <<= 1;
+    return (uint32_t)std::min<uint64_t>(s, 1ull << 31);
 }
 
 template <typename KernT, typename ParamT>
@@ -660,18 +672,20 @@ static void launch_search(const vdb_dataset* ds, const HnswSearchParams& p, uint
     }
 }
 
-// A search that could not record a neighbour in its visited set may have lost recall: fail loudly (reads and clears the
-// handle's counter; the stream is synchronised)
-void hnsw_check_overflow(const vdb_hnsw* h, cudaStream_t st) {
-    if (!h->d_overflow) return;
+// Reads and clears the handle's overflow counter (the stream is synchronised): true when a search since the last read
+// could not record a neighbour in its visited set, i.e. its results may have lost recall
+bool hnsw_take_overflow(const vdb_hnsw* h, cudaStream_t st) {
+    if (!h->d_overflow) return false;
     uint32_t v = 0;
     VDB_CUDA(cudaMemcpyAsync(&v, h->d_overflow, 4, cudaMemcpyDeviceToHost, st));
     VDB_CUDA(cudaStreamSynchronize(st));
-    if (v) {
-        VDB_CUDA(cudaMemsetAsync(h->d_overflow, 0, 4, st));
-        fail(VDB_EUNSUPPORTED, "HNSW: the visited set of a search overflowed (%u neighbours could not be recorded); results "
-                               "would lose recall, so the call fails - lower ef", v);
-    }
+    if (v) VDB_CUDA(cudaMemsetAsync(h->d_overflow, 0, 4, st));
+    return v != 0;
+}
+// a search that overflowed even a never_full_slots set (only possible past 1.8e9 rows) fails loudly
+void hnsw_check_overflow(const vdb_hnsw* h, cudaStream_t st) {
+    if (hnsw_take_overflow(h, st))
+        fail(VDB_EUNSUPPORTED, "HNSW: the visited set of a search overflowed; results would lose recall, so the call fails");
 }
 
 static HnswGraph graph_of(const vdb_hnsw* h) {
@@ -862,7 +876,7 @@ static void hnsw_insert_range(vdb_hnsw* h, const vdb_dataset* ds, uint64_t first
             sl.task_lvl = d_tlvl.as<uint32_t>();
             sl.sel = d_sel.as<uint32_t>();
             sl.selcnt = d_selcnt.as<uint32_t>();
-            {
+            auto select = [&] {
                 ProfScope prof("hnsw_select", st);
                 const size_t smem = (size_t)HN_WARPS * dimpad * 4;  // one staging row per warp
                 if (ds->dtype == VDB_F32) {
@@ -872,13 +886,28 @@ static void hnsw_insert_range(vdb_hnsw* h, const vdb_dataset* ds, uint64_t first
                     if (l2) launch_dyn(hnsw_select_kernel<uint8_t, VDB_L2SQR>, ntasks, smem, sl, st);
                     else launch_dyn(hnsw_select_kernel<uint8_t, VDB_COSINE>, ntasks, smem, sl, st);
                 }
-            }
+            };
+            select();
             // 3. arrange_links: group the back-links by (level, target), targets keep the batch order of their sources
             h_sel.resize((size_t)ntasks * M);
             h_selcnt.resize(ntasks);
+            uint32_t overflowed = 0;
+            VDB_CUDA(cudaMemcpyAsync(&overflowed, h->d_overflow, 4, cudaMemcpyDeviceToHost, st));
             VDB_CUDA(cudaMemcpyAsync(h_sel.data(), d_sel.p, (size_t)ntasks * M * 4, cudaMemcpyDeviceToHost, st));
             VDB_CUDA(cudaMemcpyAsync(h_selcnt.data(), d_selcnt.p, (size_t)ntasks * 4, cudaMemcpyDeviceToHost, st));
             VDB_CUDA(cudaStreamSynchronize(st));
+            if (overflowed) {
+                // a visited set of this batch filled up: search again with sets that cannot, and select again. The graph
+                // the search reads is unchanged: the select only wrote the lists of the batch's own nodes, which no
+                // older node links to yet
+                VDB_CUDA(cudaMemsetAsync(h->d_overflow, 0, 4, st));
+                sp.hash_mask = never_full_slots(n) - 1;
+                launch_search(ds, sp, h->d_overflow, st);
+                select();
+                VDB_CUDA(cudaMemcpyAsync(h_sel.data(), d_sel.p, (size_t)ntasks * M * 4, cudaMemcpyDeviceToHost, st));
+                VDB_CUDA(cudaMemcpyAsync(h_selcnt.data(), d_selcnt.p, (size_t)ntasks * 4, cudaMemcpyDeviceToHost, st));
+                hnsw_check_overflow(h, st);
+            }
             // (level << 32 | target, source): a stable sort by key keeps the sources of a target in batch order
             back.clear();
             for (uint32_t t = 0; t < ntasks; ++t)
@@ -951,7 +980,6 @@ vdb_hnsw* hnsw_build(const vdb_dataset* ds, uint32_t M, uint32_t ef_construction
         VDB_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
         hnsw_alloc(h, ds, M, ef_construction, h_levels, st);
         hnsw_insert_range(h, ds, 0, max_batch, st);
-        hnsw_check_overflow(h, st);
         cudaStreamDestroy(st);
     } catch (...) {
         if (st) cudaStreamDestroy(st);
@@ -1008,7 +1036,6 @@ void hnsw_append(vdb_hnsw* h, const vdb_dataset* ds, const uint32_t* new_levels,
         VDB_CUDA(cudaStreamSynchronize(st));
         hnsw_insert_range(&grown, ds, n0, max_batch, st);
         VDB_CUDA(cudaStreamSynchronize(st));
-        hnsw_check_overflow(&grown, st);
     } catch (...) {
         cudaStreamSynchronize(st);
         free_arrays(grown);
@@ -1039,7 +1066,7 @@ static void exact_topk_of(const vdb_dataset* ds, const vdb_hnsw* h, const void* 
 // knn_with_ef (:616-625) for a batch: [nq][k] keys ascending by (distance, id); distances are the cached form,
 // re-evaluated by the pair kernel that also serves vdb_gather_dist
 void hnsw_knn_keys(const vdb_dataset* ds, const vdb_hnsw* h, const void* d_queries, uint32_t nq, uint32_t k, uint32_t ef_in,
-                   uint64_t* d_keys, cudaStream_t st) {
+                   uint64_t* d_keys, cudaStream_t st, bool never_full) {
     // an index of a row-sharded set has no arrays of its own (its replicas do)
     VDB_REQUIRE(!h->rep && ds->n == h->n && ds->dim == h->dim && ds->dtype == h->dtype && ds->metric == h->metric,
                 "HNSW index was built for a different vector set");
@@ -1069,7 +1096,7 @@ void hnsw_knn_keys(const vdb_dataset* ds, const vdb_hnsw* h, const void* d_queri
     sp.qcache = qcache.as<float>();
     sp.nq = nq;
     sp.ef = ef;
-    sp.hash_mask = hash_cap_for(ef, h->M0) - 1;
+    sp.hash_mask = (never_full ? never_full_slots(h->n) : hash_cap_for(ef, h->M0)) - 1;
     sp.enter_point = (uint32_t)h->enter_point;
     sp.enter_level = (uint32_t)h->enter_level;
     sp.build = 0;
@@ -1082,7 +1109,7 @@ void hnsw_knn_keys(const vdb_dataset* ds, const vdb_hnsw* h, const void* d_queri
 // HNSWIndex::knn_pq (:672-697): the graph is walked with ADC distances, then ALL max(ef, k) results are re-scored
 // with the exact cached form and the k best by (distance, id) returned (ResultSet::pq_resort, candidate_pair.rs:102-108)
 void hnsw_knn_pq_keys(const vdb_dataset* ds, const vdb_hnsw* h, const vdb_pq* pq, const void* d_queries, uint32_t nq, uint32_t k,
-                      uint32_t ef_in, uint64_t* d_keys, cudaStream_t st) {
+                      uint32_t ef_in, uint64_t* d_keys, cudaStream_t st, bool never_full) {
     VDB_REQUIRE(!h->rep && ds->n == h->n && ds->dim == h->dim && ds->dtype == h->dtype && ds->metric == h->metric,
                 "HNSW index was built for a different vector set");
     VDB_REQUIRE(pq->metric == ds->metric, "Distance algorithm mismatch.");
@@ -1112,7 +1139,7 @@ void hnsw_knn_pq_keys(const vdb_dataset* ds, const vdb_hnsw* h, const vdb_pq* pq
     sp.qcache = qn.as<float>();  // cosine: ||q|| of the lookup table (pq_table.rs:215-221)
     sp.nq = nq;
     sp.ef = ef;
-    sp.hash_mask = hash_cap_for(ef, h->M0) - 1;
+    sp.hash_mask = (never_full ? never_full_slots(h->n) : hash_cap_for(ef, h->M0)) - 1;
     sp.enter_point = (uint32_t)h->enter_point;
     sp.enter_level = (uint32_t)h->enter_level;
     sp.build = 0;

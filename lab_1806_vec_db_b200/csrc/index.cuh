@@ -135,15 +135,17 @@ void sharded_hnsw_knn(const vdb_dataset* md, const vdb_hnsw* h, const vdb_pq* pq
 // hnsw.cu
 vdb_hnsw* hnsw_build(const vdb_dataset* ds, uint32_t M, uint32_t ef_construction, const uint32_t* h_levels, uint32_t max_batch);
 void hnsw_destroy(vdb_hnsw* h);
+bool hnsw_take_overflow(const vdb_hnsw* h, cudaStream_t st);
 void hnsw_check_overflow(const vdb_hnsw* h, cudaStream_t st);
 void hnsw_append(vdb_hnsw* h, const vdb_dataset* ds, const uint32_t* new_levels, uint32_t max_batch);
 vdb_hnsw* hnsw_from_graph(const vdb_dataset* ds, uint32_t M, uint32_t ef_construction, const uint32_t* h_levels,
                           const uint32_t* links0, const uint32_t* len0, const uint32_t* ulinks, const uint32_t* ulen,
                           int64_t enter_point, int32_t enter_level);
+// never_full: a visited set that cannot fill (the re-run of a search that overflowed)
 void hnsw_knn_keys(const vdb_dataset* ds, const vdb_hnsw* h, const void* d_queries, uint32_t nq, uint32_t k, uint32_t ef,
-                   uint64_t* d_keys, cudaStream_t st);
+                   uint64_t* d_keys, cudaStream_t st, bool never_full = false);
 void hnsw_knn_pq_keys(const vdb_dataset* ds, const vdb_hnsw* h, const vdb_pq* pq, const void* d_queries, uint32_t nq, uint32_t k,
-                      uint32_t ef, uint64_t* d_keys, cudaStream_t st);
+                      uint32_t ef, uint64_t* d_keys, cudaStream_t st, bool never_full = false);
 
 // kmeans.cu
 void kmeans_assign_exact(const void* d_rows, uint64_t n, uint64_t pitch, int dtype, int metric, uint32_t lo,

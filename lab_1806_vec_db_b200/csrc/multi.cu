@@ -1349,16 +1349,27 @@ void sharded_hnsw_knn(const vdb_dataset* md, const vdb_hnsw* h, const vdb_pq* pq
             }
         throw;
     }
-    // every replica that took part has its counter read (and cleared); a full visited set on any of them fails the call
+    // every replica that took part has its counter read (and cleared); a slice whose visited sets filled up is searched
+    // again with sets that cannot, and only a failure of that fails the call
     int code = 0;
     std::string err;
     for (Slice& x : sl) {
-        settle(x);
         try {
-            hnsw_check_overflow(rep->h[x.r], x.st);
+            VDB_CUDA(cudaSetDevice(rep->ds[x.r]->device));
+            if (hnsw_take_overflow(rep->h[x.r], x.st)) {
+                const vdb_dataset* ds = rep->ds[x.r];
+                if (pq) hnsw_knn_pq_keys(ds, rep->h[x.r], pqr->pq[x.r], x.q.p, x.cnt, k, ef, x.keys.as<uint64_t>(), x.st, true);
+                else hnsw_knn_keys(ds, rep->h[x.r], x.q.p, x.cnt, k, ef, x.keys.as<uint64_t>(), x.st, true);
+                decode_keys(x.keys.as<uint64_t>(), x.cnt, k, x.ids.as<uint64_t>(), x.dist.as<float>(), x.counts.as<uint32_t>(), x.st);
+                VDB_CUDA(cudaMemcpyAsync(ids + (size_t)x.lo * k, x.ids.p, (size_t)x.cnt * k * 8, cudaMemcpyDeviceToHost, x.st));
+                VDB_CUDA(cudaMemcpyAsync(dist + (size_t)x.lo * k, x.dist.p, (size_t)x.cnt * k * 4, cudaMemcpyDeviceToHost, x.st));
+                VDB_CUDA(cudaMemcpyAsync(counts + x.lo, x.counts.p, (size_t)x.cnt * 4, cudaMemcpyDeviceToHost, x.st));
+                hnsw_check_overflow(rep->h[x.r], x.st);
+            }
         } catch (const Error& e) {
             if (!code) code = e.code, err = e.what();
         }
+        settle(x);
     }
     if (code) throw Error(code, err);
 }

@@ -104,6 +104,10 @@ struct PairLess {
 struct ResultSet {
     size_t k;
     std::set<Pair, PairLess> s;
+    /* adds to a full set whose distance equals the last entry's: the reference keeps the older entry whatever the
+     * ids, where a selection of the k smallest (distance, id) keys may keep the newer one. Counted so that tests can
+     * tell an exact distance tie from a real difference. */
+    size_t ties = 0;
     explicit ResultSet(size_t k_) : k(k_) {}
     bool add(Pair p) { /* :61-74 */
         if (s.size() < k) {
@@ -112,11 +116,13 @@ struct ResultSet {
         }
         if (!s.empty()) {
             auto last = std::prev(s.end());
-            if (cmp_of(p.d, last->d) < 0) { /* strict, distance only */
+            const int c = cmp_of(p.d, last->d);
+            if (c < 0) { /* strict, distance only */
                 s.erase(last);
                 s.insert(p);
                 return true;
             }
+            if (c == 0) ++ties;
         }
         return false;
     }
@@ -540,7 +546,8 @@ template <class T> struct Hnsw {
         len[v][level] = lk.size();
         std::copy(lk.begin(), lk.end(), links(v, level));
     }
-    void add(size_t idx, size_t level) { /* push_init :241-256 + add :538-572 */
+    uint64_t build_ties = 0; /* tie events (ResultSet::ties) of every candidate search of the build */
+    void push_init(size_t idx, size_t level) { /* :241-256: a node without links */
         level0.resize((idx + 1) * max_m0, 0);
         other.emplace_back(m * level, 0u);
         len.emplace_back(level + 1, (size_t)0);
@@ -548,16 +555,21 @@ template <class T> struct Hnsw {
         const T* v = rows + idx * dim;
         cache.push_back(metric == ORC_L2SQR ? dot(v, v, dim) : vec_norm(v, dim));
         n = idx + 1;
+    }
+    void add(size_t idx, size_t level) { /* push_init :241-256 + add :538-572 */
+        push_init(idx, level);
         if (enter_point < 0) {
             enter_level = (long)level;
             enter_point = (long)idx;
             return;
         }
+        const T* v = rows + idx * dim;
         const float qc = cache[idx];
         auto dist_fn = [&](size_t i) { return d_cached(i, v, qc); };
         size_t cur = (long)level < enter_level ? greedy(level, dist_fn) : (size_t)enter_point;
         for (long l = std::min<long>((long)level, enter_level); l >= 0; --l) {
             ResultSet cand = search_on_level(cur, (size_t)l, ef_c, dist_fn);
+            build_ties += cand.ties;
             cur = cand.s.begin()->i;
             auto nb = heuristic(cand.s, m); /* connect_new_links :226-239 */
             for (size_t j = 0; j < nb.size(); ++j) links(idx, (size_t)l)[j] = (uint32_t)nb[j].i;
@@ -567,6 +579,72 @@ template <class T> struct Hnsw {
         if ((long)level > enter_level) {
             enter_level = (long)level;
             enter_point = (long)idx;
+        }
+    }
+    /* The device build (hnsw.cu, hnsw_insert_range) restated: rows [n, end) are inserted a batch at a time, batch
+     * size min(max(1, done / m), max_batch, rows left). Every node of a batch searches the graph as it stood when the
+     * batch began; on each level the entry of the next level is the graph search's best, taken before the candidates
+     * are merged with the earlier nodes of the batch that live on that level. Then every (node, level) selects its
+     * links (at most m, level 0 too), then the back-links are applied grouped by (level, target), the sources of a
+     * target in task order (node, then level upwards). The enter point moves after the batch. With max_batch = 1 this
+     * is `add` row by row. */
+    void insert_batched(size_t end, const uint32_t* levels, size_t max_batch) {
+        size_t done = n;
+        if (done >= end) return;
+        if (enter_point < 0) { /* the first vector becomes the enter point (:543-551) */
+            add(done, levels[done]);
+            ++done;
+        }
+        while (done < end) {
+            const size_t b = std::min(std::min(std::max<size_t>(1, done / m), max_batch), end - done);
+            const size_t first = done;
+            for (size_t i = first; i < first + b; ++i) push_init(i, levels[i]);
+            struct Task {
+                size_t node, level;
+                std::vector<Pair> sel;
+            };
+            std::vector<Task> tasks;
+            std::vector<std::vector<ResultSet>> cands(b); /* [node][level] */
+            for (size_t i = first; i < first + b; ++i) {
+                const T* v = rows + i * dim;
+                const float qc = cache[i];
+                auto dist_fn = [&](size_t x) { return d_cached(x, v, qc); };
+                const size_t level = levels[i];
+                size_t cur = (long)level < enter_level ? greedy(level, dist_fn) : (size_t)enter_point;
+                const long top = std::min<long>((long)level, enter_level);
+                cands[i - first].assign((size_t)top + 1, ResultSet(0));
+                for (long l = top; l >= 0; --l) {
+                    ResultSet cand = search_on_level(cur, (size_t)l, ef_c, dist_fn);
+                    cur = cand.s.begin()->i;
+                    for (size_t j = first; j < i; ++j) /* brute force among the batch (:431-437) */
+                        if ((long)levels[j] >= l) cand.add(Pair{dist_fn(j), j});
+                    build_ties += cand.ties;
+                    cands[i - first][(size_t)l] = std::move(cand);
+                }
+            }
+            for (size_t i = first; i < first + b; ++i)
+                for (size_t l = 0; l < cands[i - first].size(); ++l) {
+                    Task t{i, l, heuristic(cands[i - first][l].s, m)};
+                    for (size_t j = 0; j < t.sel.size(); ++j) links(i, l)[j] = (uint32_t)t.sel[j].i;
+                    len[i][l] = t.sel.size();
+                    tasks.push_back(std::move(t));
+                }
+            struct Back {
+                size_t level, target, source;
+            };
+            std::vector<Back> back;
+            for (const Task& t : tasks)
+                for (const Pair& p : t.sel) back.push_back(Back{t.level, p.i, t.node});
+            std::stable_sort(back.begin(), back.end(), [](const Back& a, const Back& c) {
+                return a.level != c.level ? a.level < c.level : a.target < c.target;
+            });
+            for (const Back& e : back) arrange(e.target, e.level, e.source);
+            for (size_t i = first; i < first + b; ++i)
+                if ((long)levels[i] > enter_level) {
+                    enter_level = (long)levels[i];
+                    enter_point = (long)i;
+                }
+            done += b;
         }
     }
 };
@@ -758,6 +836,36 @@ void* orc_hnsw_build(const void* rows, size_t n, size_t dim, int dtype, int metr
     });
     return nullptr;
 }
+/* The device build's batch pipeline (Hnsw::insert_batched): rows [0, n0) are inserted as one build, then rows [n0, n)
+ * as an append onto that graph (batch sizes restart from done = n0, like vdb_hnsw_append). n0 = 0: one build. */
+void* orc_hnsw_build_batched(const void* rows, size_t n, size_t dim, int dtype, int metric, size_t m, size_t ef_construction,
+                             const uint32_t* levels, size_t max_batch, size_t n0) {
+    if (max_batch == 0 || n0 > n) return nullptr;
+    D1(dtype, {
+        auto* h = new Hnsw<T>();
+        h->rows = (const T*)rows;
+        h->dim = dim;
+        h->m = m;
+        h->max_m0 = 2 * m;
+        h->ef_c = std::max(ef_construction, 2 * m);
+        h->metric = metric;
+        h->insert_batched(n0, levels, max_batch);
+        h->insert_batched(n, levels, max_batch);
+        return (void*)h;
+    });
+    return nullptr;
+}
+uint64_t orc_hnsw_build_ties(const void* handle, int dtype) {
+    D1(dtype, return ((const Hnsw<T>*)handle)->build_ties);
+    return 0;
+}
+int orc_hnsw_enter(const void* handle, int dtype, long* enter_point, long* enter_level) {
+    D1(dtype, {
+        *enter_point = ((const Hnsw<T>*)handle)->enter_point;
+        *enter_level = ((const Hnsw<T>*)handle)->enter_level;
+    });
+    return 0;
+}
 /* An index whose graph was built elsewhere (HNSWIndex deserialisation, hnsw_index.rs:641-668, followed by
  * init_dist_cache_after_load :371-379): levels[n], level-0 links [n][2m] + lengths, upper levels per node in row order
  * ([sum(levels)][m] + lengths). Lets the CPU search walk the very graph the GPU built. */
@@ -799,11 +907,12 @@ void* orc_hnsw_from_graph(const void* rows, size_t n, size_t dim, int dtype, int
     return nullptr;
 }
 int orc_hnsw_knn(const void* handle, int dtype, const void* queries, size_t nq, size_t k, size_t ef, uint64_t* ids,
-                 float* dists, uint32_t* counts, int nthreads) {
+                 float* dists, uint32_t* counts, int nthreads, uint32_t* ties) {
     D1(dtype, {
         const auto* h = (const Hnsw<T>*)handle;
         parallel_for(nq, nthreads, [&](size_t q) {
             const T* qv = (const T*)queries + q * h->dim;
+            if (ties) ties[q] = 0;
             if (h->n == 0) {
                 counts[q] = 0;
                 return;
@@ -813,13 +922,15 @@ int orc_hnsw_knn(const void* handle, int dtype, const void* queries, size_t nq, 
             size_t ep = h->greedy(0, dist_fn);
             ResultSet r = h->search_on_level(ep, 0, std::max(ef, k), dist_fn);
             counts[q] = (uint32_t)emit(r, k, ids + q * k, dists + q * k);
+            if (ties) ties[q] = (uint32_t)r.ties;
         });
     });
     return 0;
 }
 /* HNSWIndex::knn_pq (hnsw_index.rs:672-697): graph walk with ADC distances, then pq_resort with dist_with_cache */
 int orc_hnsw_knn_pq(const void* handle, int dtype, const void* queries, size_t nq, size_t k, size_t ef, const uint8_t* codes,
-                    const void* codebooks, size_t m, size_t n_bits, uint64_t* ids, float* dists, uint32_t* counts, int nthreads) {
+                    const void* codebooks, size_t m, size_t n_bits, uint64_t* ids, float* dists, uint32_t* counts, int nthreads,
+                    uint32_t* ties) {
     D1(dtype, {
         const auto* h = (const Hnsw<T>*)handle;
         const size_t kc = (size_t)1 << n_bits;
@@ -828,6 +939,7 @@ int orc_hnsw_knn_pq(const void* handle, int dtype, const void* queries, size_t n
         pq_dist_cache<T>(h->dim, h->metric, (const T*)codebooks, m, n_bits, dcache.data());
         parallel_for(nq, nthreads, [&](size_t q) {
             const T* qv = (const T*)queries + q * h->dim;
+            if (ties) ties[q] = 0;
             if (h->n == 0) {
                 counts[q] = 0;
                 return;
@@ -842,6 +954,7 @@ int orc_hnsw_knn_pq(const void* handle, int dtype, const void* queries, size_t n
             ResultSet rs(k);
             for (const Pair& p : r.s) rs.add({h->d_cached(p.i, qv, qc), p.i});
             counts[q] = (uint32_t)emit(rs, k, ids + q * k, dists + q * k);
+            if (ties) ties[q] = (uint32_t)(r.ties + rs.ties);   /* the walk's and pq_resort's */
         });
     });
     return 0;

@@ -116,10 +116,20 @@ void* orc_hnsw_build(const void* rows, size_t n, size_t dim, int dtype, int metr
 void* orc_hnsw_from_graph(const void* rows, size_t n, size_t dim, int dtype, int metric, size_t m, size_t ef_construction,
                           const uint32_t* levels, const uint32_t* links0, const uint32_t* len0, const uint32_t* ulinks,
                           const uint32_t* ulen, long enter_point, long enter_level);
+/* the batch pipeline of the device build (hnsw.cu hnsw_insert_range): a build of rows [0, n0), then an append of
+ * rows [n0, n) onto it; n0 = 0 is one build. max_batch = 1 gives orc_hnsw_build's graph. */
+void* orc_hnsw_build_batched(const void* rows, size_t n, size_t dim, int dtype, int metric, size_t m, size_t ef_construction,
+                             const uint32_t* levels, size_t max_batch, size_t n0);
+/* Tie events: adds to a full ResultSet with a distance equal to its last entry's (candidate_pair.rs:61-74 keeps the
+ * older entry; a k-smallest selection by (distance, id) may not). Of a whole build: */
+uint64_t orc_hnsw_build_ties(const void* handle, int dtype);
+int orc_hnsw_enter(const void* handle, int dtype, long* enter_point, long* enter_level);
+/* ties (may be NULL): [nq] tie events of each query's walk (and, for knn_pq, of its pq_resort) */
 int orc_hnsw_knn(const void* handle, int dtype, const void* queries, size_t nq, size_t k, size_t ef, uint64_t* ids,
-                 float* dists, uint32_t* counts, int nthreads);
+                 float* dists, uint32_t* counts, int nthreads, uint32_t* ties);
 int orc_hnsw_knn_pq(const void* handle, int dtype, const void* queries, size_t nq, size_t k, size_t ef, const uint8_t* codes,
-                    const void* codebooks, size_t m, size_t n_bits, uint64_t* ids, float* dists, uint32_t* counts, int nthreads);
+                    const void* codebooks, size_t m, size_t n_bits, uint64_t* ids, float* dists, uint32_t* counts, int nthreads,
+                    uint32_t* ties);
 int orc_hnsw_links0(const void* handle, int dtype, uint32_t* links0, uint32_t* len0);
 int orc_hnsw_upper(const void* handle, int dtype, uint32_t* ulinks, uint32_t* ulen);
 void orc_hnsw_free(void* handle, int dtype);

@@ -263,8 +263,19 @@ def recall(gnd, pred):
     return lib().orc_recall(_p(gnd), gnd.size, _p(pred), pred.size)
 
 
+_KNN_ARGS = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p,
+             C.c_int, C.c_void_p]
+_KNN_PQ_ARGS = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_void_p, C.c_void_p, C.c_size_t,
+                C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+
+
 class HnswOracle:
-    """Single-thread restatement of HNSWIndex (sequential add of every row, knn_with_ef); recall yardstick."""
+    """Single-thread restatement of HNSWIndex (sequential add of every row, knn_with_ef); recall yardstick.
+
+    Tie events: an add to a full result set with a distance equal to its last entry's. The reference keeps the older
+    entry whatever the ids, a selection of the smallest (distance, id) keys may keep the newer one; on data where every
+    distance is exact that is the only way two correct walks over the same graph can differ. `build_ties` counts them
+    over a build, `knn(..., ties=True)` per query."""
 
     def __init__(self, base, metric, m, ef_construction, levels):
         self.base = _c(base)
@@ -274,8 +285,6 @@ class HnswOracle:
         f = lib().orc_hnsw_build
         f.restype = C.c_void_p
         f.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_void_p]
-        lib().orc_hnsw_knn.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_void_p,
-                                       C.c_void_p, C.c_void_p, C.c_int]
         lib().orc_hnsw_links0.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         lib().orc_hnsw_free.argtypes = [C.c_void_p, C.c_int]
         lib().orc_hnsw_free.restype = None
@@ -296,8 +305,6 @@ class HnswOracle:
         f.restype = C.c_void_p
         f.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_void_p, C.c_void_p,
                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_long, C.c_long]
-        lib().orc_hnsw_knn.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_void_p,
-                                       C.c_void_p, C.c_void_p, C.c_int]
         lib().orc_hnsw_free.argtypes = [C.c_void_p, C.c_int]
         lib().orc_hnsw_free.restype = None
         ul = self._keep[2] if self._keep[2].size else np.zeros(1, np.uint32)
@@ -307,27 +314,67 @@ class HnswOracle:
                               int(enter_point), int(enter_level)))
         return self
 
-    def knn(self, queries, k, ef, nthreads=1):
+    @classmethod
+    def batched(cls, base, metric, m, ef_construction, levels, max_batch, n0=0):
+        """The device build's batch pipeline (orc_hnsw_build_batched): a build of rows [0, n0), then an append of the
+        rest onto it (n0 = 0: one build of every row)."""
+        self = cls.__new__(cls)
+        self.base = _c(base)
+        self.dt = _dt(self.base)
+        self.levels = _c(levels, np.uint32)
+        self.m = m
+        f = lib().orc_hnsw_build_batched
+        f.restype = C.c_void_p
+        f.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_void_p, C.c_size_t,
+                      C.c_size_t]
+        h = f(_p(self.base), self.base.shape[0], self.base.shape[1], self.dt, _METRIC[metric], m, ef_construction,
+              _p(self.levels), max_batch, n0)
+        assert h, "orc_hnsw_build_batched: max_batch must be positive and n0 <= n"
+        self.h = C.c_void_p(h)
+        return self
+
+    @property
+    def build_ties(self):
+        f = lib().orc_hnsw_build_ties
+        f.restype = C.c_uint64
+        f.argtypes = [C.c_void_p, C.c_int]
+        return int(f(self.h, self.dt))
+
+    @property
+    def enter_point(self):
+        """(enter point, enter level), like HNSWIndex.enter_point"""
+        f = lib().orc_hnsw_enter
+        f.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+        ep, el = C.c_long(-1), C.c_long(-1)
+        f(self.h, self.dt, C.byref(ep), C.byref(el))
+        return int(ep.value), int(el.value)
+
+    def knn(self, queries, k, ef, nthreads=1, ties=False):
+        """(ids, dist, counts), and with ties=True the tie events of every query's walk as a fourth array"""
         q = _c(queries)
         nq = q.shape[0]
         ids = np.zeros((nq, k), np.uint64)
         dd = np.zeros((nq, k), np.float32)
         cnt = np.zeros(nq, np.uint32)
-        lib().orc_hnsw_knn(self.h, self.dt, _p(q), C.c_size_t(nq), C.c_size_t(k), C.c_size_t(ef), _p(ids), _p(dd),
-                           _p(cnt), nthreads)
-        return ids, dd, cnt
+        tie = np.zeros(max(nq, 1), np.uint32)
+        f = lib().orc_hnsw_knn
+        f.argtypes = _KNN_ARGS
+        f(self.h, self.dt, _p(q), nq, k, ef, _p(ids), _p(dd), _p(cnt), nthreads, _p(tie))
+        return (ids, dd, cnt, tie[:nq]) if ties else (ids, dd, cnt)
 
-    def knn_pq(self, queries, k, ef, codes, codebooks, m, n_bits, nthreads=1):
+    def knn_pq(self, queries, k, ef, codes, codebooks, m, n_bits, nthreads=1, ties=False):
+        """(ids, dist, counts), and with ties=True the tie events of every query's walk and resort"""
         q, codes, codebooks = _c(queries), _c(codes, np.uint8), _c(codebooks)
         nq = q.shape[0]
         ids = np.zeros((nq, k), np.uint64)
         dd = np.zeros((nq, k), np.float32)
         cnt = np.zeros(nq, np.uint32)
+        tie = np.zeros(max(nq, 1), np.uint32)
         f = lib().orc_hnsw_knn_pq
-        f.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_void_p, C.c_void_p, C.c_size_t,
-                      C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
-        f(self.h, self.dt, _p(q), nq, k, ef, _p(codes), _p(codebooks), m, n_bits, _p(ids), _p(dd), _p(cnt), nthreads)
-        return ids, dd, cnt
+        f.argtypes = _KNN_PQ_ARGS
+        f(self.h, self.dt, _p(q), nq, k, ef, _p(codes), _p(codebooks), m, n_bits, _p(ids), _p(dd), _p(cnt), nthreads,
+          _p(tie))
+        return (ids, dd, cnt, tie[:nq]) if ties else (ids, dd, cnt)
 
     def links0(self):
         n = self.base.shape[0]

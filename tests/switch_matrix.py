@@ -72,8 +72,8 @@ OTHER = {
     "VDB_SCAN_FUSE": ("call", "tests/test_flat_gpu.py::test_fused_scan_tail_equals_the_separate_merge"),
     "VDB_PQ_NO_DECODE": ("call", "tests/test_index_gpu.py::test_pq_decoded_contraction_large_shard"),
     "VDB_MG_GLOBAL_PRUNE": ("call", "tests/test_multi_gpu.py::test_global_pruning_bound_changes_no_bit_and_gathers_fewer_rows"),
-    "VDB_HNSW_HASH_SLOTS": ("process", "test hook: forces the visited-set size; "
-                                       "tests/test_hnsw_gpu.py::test_a_full_visited_set_is_an_error_not_a_silent_loss"),
+    "VDB_HNSW_HASH_SLOTS": ("process", "test hook: forces the first visited-set size of every search; "
+                                       "tests/test_hnsw_gpu.py::test_a_full_visited_set_is_searched_again_not_a_silent_loss"),
     "VDB_MG_TRACE": ("process", "diagnostic print of the sharded search's host phase times; selects no kernel"),
 }
 
