@@ -315,53 +315,21 @@ uint32_t kmeans_lloyd(const void* d_rows, uint64_t n, uint64_t pitch, int dtype,
 }
 
 // ---- k-means++ weights: w[i] = min(w[i], d(c, v_i)) ----------------------------------------------------
-template <typename T, int METRIC>
-__global__ void pp_weights_kernel(const T* __restrict__ rows, uint64_t n, uint64_t pitch, uint32_t lo, uint32_t d,
-                                  const T* __restrict__ c, float* __restrict__ w) {
-    const int lane = threadIdx.x & 31;
-    const uint64_t warp = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
-    for (uint64_t i = warp; i < n; i += nwarps) {
-        float s0 = 0.f, s1 = 0.f, s2 = 0.f;
-        for (uint32_t j = lane; j < d; j += 32) {
-            const float x = to_f32(rows[i * pitch + lo + j]), y = to_f32(c[j]);
-            if (METRIC == VDB_L2SQR) {
-                const float df = y - x;
-                s0 = fmaf(df, df, s0);
-            } else {
-                s0 = fmaf(x, y, s0);
-                s1 = fmaf(x, x, s1);
-                s2 = fmaf(y, y, s2);
-            }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            s0 += __shfl_xor_sync(0xffffffffu, s0, o);
-            s1 += __shfl_xor_sync(0xffffffffu, s1, o);
-            s2 += __shfl_xor_sync(0xffffffffu, s2, o);
-        }
-        if (lane == 0) {
-            const float dd = METRIC == VDB_L2SQR ? s0 : 1.0f - s0 / fmaxf(sqrtf(s2) * sqrtf(s1), 1e-10f);
-            w[i] = fminf(w[i], dd);
-        }
-    }
+// d(c, v_i) must be the reference's sequential f32 chain (k_means.rs:76): every weight moves a WeightedIndex boundary, so
+// a last-bit difference can change a pick. The assignment kernel with the single centroid c computes exactly that chain
+// (rows staged through shared memory with coalesced loads); its all_dist output is folded into w here.
+__global__ void fmin_into_kernel(const float* __restrict__ d, uint64_t n, float* __restrict__ w) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+        w[i] = fminf(w[i], d[i]);   // f32::min: a NaN operand yields the other one
 }
 
 void kmeans_pp_weights(const void* d_rows, uint64_t n, uint64_t pitch, int dtype, int metric, uint32_t lo,
                        uint32_t d, const void* d_c, float* d_w, cudaStream_t st) {
     if (n == 0) return;
-    const uint32_t grid = (uint32_t)std::min<uint64_t>(ceil_div<uint64_t>(n, 8), (uint64_t)sm_count() * 16);
-    if (dtype == VDB_F32) {
-        if (metric == VDB_L2SQR)
-            pp_weights_kernel<float, VDB_L2SQR><<<grid, 256, 0, st>>>((const float*)d_rows, n, pitch, lo, d, (const float*)d_c, d_w);
-        else
-            pp_weights_kernel<float, VDB_COSINE><<<grid, 256, 0, st>>>((const float*)d_rows, n, pitch, lo, d, (const float*)d_c, d_w);
-    } else {
-        if (metric == VDB_L2SQR)
-            pp_weights_kernel<uint8_t, VDB_L2SQR><<<grid, 256, 0, st>>>((const uint8_t*)d_rows, n, pitch, lo, d, (const uint8_t*)d_c, d_w);
-        else
-            pp_weights_kernel<uint8_t, VDB_COSINE><<<grid, 256, 0, st>>>((const uint8_t*)d_rows, n, pitch, lo, d, (const uint8_t*)d_c, d_w);
-    }
+    DevBuf best(n * 8, st), dist(n * 4, st);
+    kmeans_assign_exact(d_rows, n, pitch, dtype, metric, lo, d, d_c, 1, best.as<uint64_t>(), nullptr, dist.as<float>(), st);
+    fmin_into_kernel<<<(uint32_t)std::min<uint64_t>(ceil_div<uint64_t>(n, 256), (uint64_t)sm_count() * 8), 256, 0, st>>>(
+        dist.as<float>(), n, d_w);
     VDB_LAUNCHED();
 }
 

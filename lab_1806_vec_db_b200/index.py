@@ -271,7 +271,7 @@ def k_means_init_reference_stream(rows_host, config: KMeansConfig, rng):
     """k-means++ (k_means.rs:61-87) under the reference's OWN random stream (`rand_compat.StdRng`: rand 0.8.5 restated,
     parity with the crate unpinned - see that module): gen_range for the first pick, per round the f32 WeightedIndex over
     the weights the GPU updates (`vdb_kmeans_pp_weights`: w[i] = min(w[i], d(c, v_i)) with the reference's sequential f32
-    distance) and the eagerly drawn fallback. Rows stay on the host (the weights call stages them)."""
+    distance, bit for bit) and the eagerly drawn fallback. Rows stay on the host (the weights call stages them)."""
     from .rand_compat import k_means_init_indices
     rows = np.ascontiguousarray(rows_host)
     n, dim = rows.shape

@@ -397,6 +397,15 @@ struct SplitMix {
     size_t below(size_t n) { return (size_t)(uniform() * (double)n) % n; }
 };
 
+/* ---- k_means.rs:75-77: the k-means++ weight update w[i] = min(w[i], d(c, v_i[lo:hi])) -------- */
+template <class T>
+void kmeans_pp_weights(const T* rows, size_t n, size_t dim, int metric, const T* c, size_t lo, size_t hi, float* w,
+                       int nthreads) {
+    parallel_chunks(n, nthreads, 256, [&](size_t i) {
+        w[i] = std::fmin(w[i], dist(c, rows + i * dim + lo, hi - lo, metric)); /* d(c, v) :76, f32::min */
+    });
+}
+
 /* ---- k_means.rs:61-87: k-means++ (structure only; draws are not the reference's) ----------- */
 template <class T>
 void kmeans_pp(const T* rows, size_t n, size_t dim, int metric, size_t k, size_t lo, size_t hi,
@@ -407,12 +416,10 @@ void kmeans_pp(const T* rows, size_t n, size_t dim, int metric, size_t k, size_t
     std::memcpy(cent, rows + first * dim + lo, d * sizeof(T));
     std::vector<float> w(n, std::numeric_limits<float>::infinity());
     for (size_t idx = 1; idx < k; ++idx) {
-        const T* prev = cent + (idx - 1) * d;
+        kmeans_pp_weights(rows, n, dim, metric, cent + (idx - 1) * d, lo, hi, w.data(), 1);
         double total = 0.0;
         bool ok = true;
         for (size_t i = 0; i < n; ++i) {
-            float dd = dist(prev, rows + i * dim + lo, d, metric); /* d(c, v) :76 */
-            w[i] = std::fmin(w[i], dd);
             if (!(w[i] >= 0.0f) || std::isinf(w[i])) ok = false; /* WeightedIndex rejects <0 / NaN */
             total += w[i];
         }
@@ -728,6 +735,12 @@ int orc_kmeans_pp_init(const void* rows, size_t n, size_t dim, int dtype, int me
                        size_t sel_lo, size_t sel_hi, uint64_t seed, void* centroids) {
     if (n == 0 || k == 0) return 1;
     D1(dtype, kmeans_pp((const T*)rows, n, dim, metric, k, sel_lo, sel_hi, seed, (T*)centroids));
+    return 0;
+}
+int orc_kmeans_pp_weights(const void* rows, size_t n, size_t dim, int dtype, int metric, const void* c, size_t sel_lo,
+                          size_t sel_hi, float* w, int nthreads) {
+    if (sel_lo > sel_hi || sel_hi > dim) return 1;
+    D1(dtype, kmeans_pp_weights((const T*)rows, n, dim, metric, (const T*)c, sel_lo, sel_hi, w, nthreads));
     return 0;
 }
 

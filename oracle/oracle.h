@@ -71,6 +71,10 @@ int orc_kmeans_lloyd(const void* rows, size_t n, size_t dim, int dtype, int metr
  * writes [k, sel_hi-sel_lo] initial centroids. */
 int orc_kmeans_pp_init(const void* rows, size_t n, size_t dim, int dtype, int metric,
                        size_t k, size_t sel_lo, size_t sel_hi, uint64_t seed, void* centroids);
+/* k_means.rs:75-77: the k-means++ weight update w[i] = min(w[i], d(c, rows[i][sel_lo:sel_hi])) for i < n, c of
+ * length sel_hi-sel_lo, the rows split across nthreads. kmeans_pp uses this same update. */
+int orc_kmeans_pp_weights(const void* rows, size_t n, size_t dim, int dtype, int metric, const void* c,
+                          size_t sel_lo, size_t sel_hi, float* w, int nthreads);
 
 /* pq_table.rs:66-91,178-181. codebooks: m groups concatenated, group g = [kc, len_g] of dtype,
  * kc = 1<<n_bits. codes out: [n, encoded_dim]. */

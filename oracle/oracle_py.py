@@ -49,6 +49,7 @@ def lib():
         L.orc_kmeans_assign.argtypes = [vp, sz, sz, i32, i32, vp, sz, sz, sz, vp, i32]
         L.orc_kmeans_lloyd.argtypes = [vp, sz, sz, i32, i32, vp, sz, sz, sz, sz, f]
         L.orc_kmeans_pp_init.argtypes = [vp, sz, sz, i32, i32, sz, sz, sz, C.c_uint64, vp]
+        L.orc_kmeans_pp_weights.argtypes = [vp, sz, sz, i32, i32, vp, sz, sz, vp, i32]
         L.orc_pq_encode.argtypes = [vp, sz, sz, i32, i32, vp, sz, sz, vp, i32]
         L.orc_pq_lookup.argtypes = [vp, sz, i32, i32, vp, sz, sz, vp, vp]
         L.orc_pq_dist_cache.argtypes = [sz, i32, i32, vp, sz, sz, vp]
@@ -154,6 +155,19 @@ def kmeans_pp_init(rows, k, metric, seed, sel=None):
     rc = lib().orc_kmeans_pp_init(_p(rows), n, dim, _dt(rows), _METRIC[metric], k, lo, hi, seed, _p(cent))
     assert rc == 0
     return cent
+
+
+def kmeans_pp_weights(rows, c, metric, w, sel=None, nthreads=1):
+    """The k-means++ weight update (k_means.rs:75-77): returns min(w, d(c, rows[:, lo:hi])) as a new f32 array."""
+    rows, c = _c(rows), _c(c)
+    n, dim = rows.shape
+    lo, hi = sel if sel is not None else (0, dim)
+    assert c.dtype == rows.dtype and c.size == hi - lo
+    out = np.array(w, dtype=np.float32, order="C", copy=True)
+    assert out.shape == (n,)
+    rc = lib().orc_kmeans_pp_weights(_p(rows), n, dim, _dt(rows), _METRIC[metric], _p(c), lo, hi, _p(out), nthreads)
+    assert rc == 0, "kmeans_pp_weights: invalid selected range"
+    return out
 
 
 def find_n_nearest(v, centroids, n_probes, metric):

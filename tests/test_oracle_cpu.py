@@ -150,6 +150,31 @@ def test_kmeans_on_real_set_property(fixtures, oracle):
     assert oracle.kmeans_assign(v.reshape(1, -1), cent, "l2sqr", sel=(0, 5))[0] == 1
 
 
+@pytest.mark.parametrize("metric", ["l2sqr", "cosine"])
+@pytest.mark.parametrize("dtype", ["f32", "u8"])
+def test_kmeans_pp_weights_equals_numpy_emulation(fixtures, oracle, metric, dtype):
+    """k_means.rs:75-77: w[i] = min(w[i], d(c, v_i)) on the whole row and on a window with lo > 0, two rounds (the second
+    keeps the smaller old weight for part of the rows), split across threads: bit for bit the numpy emulation's
+    sequential f32 distance. A row equal to the centroid gets weight 0."""
+    import sys
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+    import np_emul as E
+    base = fixtures["base"][:300]
+    rows = base if dtype == "f32" else np.clip(np.rint(base * 255.0), 0, 255).astype(np.uint8)
+    for lo, hi in ((0, rows.shape[1]), (37, 170)):
+        sub = rows[:, lo:hi]
+        want = np.full(len(rows), np.inf, np.float32)
+        got = want.copy()
+        for c in (11, 250):
+            d = E.distance(np.broadcast_to(sub[c], sub.shape), sub, metric)
+            want = np.fmin(want, d).astype(np.float32)
+            got = oracle.kmeans_pp_weights(rows, sub[c], metric, got, sel=(lo, hi), nthreads=4)
+            assert (bits(got) == bits(want)).all(), (lo, hi, c)
+            assert got[c] == 0.0 or metric == "cosine"
+        kept = bits(got) != bits(E.distance(np.broadcast_to(sub[250], sub.shape), sub, metric))
+        assert kept.any() and not kept.all()
+
+
 def test_lloyd_empty_cluster_and_u8_cast(oracle):
     """k_means.rs:131-137 (empty cluster keeps its centroid) and scalar.rs:22-37 (`as u8`)."""
     rows = np.array([[0, 0], [2, 0], [0, 2], [2, 2]], np.uint8)
